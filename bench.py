@@ -3,7 +3,7 @@
 8778-pair 10-decoder eVAE energy optimisation).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision f16|f16x3|tf32|fp32]
-                    [--config 3|5|2]
+                    [--config 3|5|2] [--dump-outputs DIR]
 
 A "step" is one Adam step of EVERY curve of the workload (= n_curves spline-steps): spline
 evaluation, all-decoder forward + input-gradient backward, MC pair energy, Adam -- one pass of
@@ -279,6 +279,14 @@ def cpu_reference_rate(cfg, steps, warmup, budget_s):
     return rate, cores, kind, what
 
 
+def write_outputs(out_dir: Path, outputs):
+    """<out_dir>/<name>.npy, float32 as computed, every curve: energy [N] and omega / adam_m / adam_v
+    [N, n_poly + 1, 2] -- 1.1 MB for configs 2 and 3, 22 MB for config 5."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, x in outputs.items():
+        np.save(out_dir / f"{name}.npy", x.cpu().numpy())
+
+
 def workload_config(cfg, gpus, where, extra=None):
     d = {"workload": cfg["name"], "n_curves": cfg["N"], "T": cfg["T"], "K": cfg["K"], "M": cfg["M"],
          "n_poly": cfg["n_poly"], "weights": cfg["weights"],
@@ -354,7 +362,8 @@ def run_gpu_arm(args):
         return vlg_b200.GeodesicSplineBatch(h_a.to(dev), h_b.to(dev), basis, h_om.to(dev), n_poly)
 
     def timed_steps(prec, nsteps, nwarm):
-        """K steps with the curve state resident in HBM; returns (ms over the region, ms inside kernels, launches)."""
+        """K steps with the curve state resident in HBM; returns (ms over the region, ms inside kernels, launches,
+        the launch function, what the last timed step handed back: {energy, omega, adam_m, adam_v})."""
         model = fresh_model()
 
         def launch(ns):
@@ -371,13 +380,16 @@ def run_gpu_arm(args):
             flush.fill_(done & 0xFF)
             k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             k0.record()
-            launch(ns)
+            energy = launch(ns)
             k1.record()
             events.append((k0, k1))
             done += ns
         ev1.record()
         barrier()
-        return ev0.elapsed_time(ev1), sum(x.elapsed_time(y) for x, y in events), len(events), launch
+        # copies: later launches (the same-load tail below) keep updating the model in place
+        outputs = {"energy": energy.clone(), "omega": model.omega.clone(), "adam_m": model.adam_m.clone(),
+                   "adam_v": model.adam_v.clone()}
+        return ev0.elapsed_time(ev1), sum(x.elapsed_time(y) for x, y in events), len(events), launch, outputs
 
     # clocks are sampled (nvidia-smi, 100 ms period) from the warm-up on: the timed region of a sharded run can
     # be shorter than one sampling period, so the same load is kept up before and after it (see below)
@@ -385,7 +397,7 @@ def run_gpu_arm(args):
     sampler.start()
 
     # ---- value: K steps, state resident in HBM ----
-    ms_total, kernel_ms, launches, launch = timed_steps(precision, args.steps, max(args.warmup, 3))
+    ms_total, kernel_ms, launches, launch, outputs = timed_steps(precision, args.steps, max(args.warmup, 3))
     # untimed tail under the same load until the sampler has seen the GPU busy at least three times
     t_tail = time.time()
     while len(sampler.rows) < 3 and time.time() - t_tail < 2.0:
@@ -440,10 +452,15 @@ def run_gpu_arm(args):
             if prec == precision or (K == 1 and prec in ("f16", "tf32")):
                 continue
             ns = args.steps if prec != "fp32" else max(1, min(args.steps, 2))
-            ms, kms, _, _ = timed_steps(prec, ns, 2)
+            ms, kms, _, _, _ = timed_steps(prec, ns, 2)
             other[prec] = {"value": N * ns / (ms * 1e-3), "unit": "spline-steps/s", "steps": ns,
                            "roofline_frac": N * ns * T * K * FLOP_PER_POINT_DECODER / (kms * 1e-3) / 1e12 / measured_peak()[0],
                            "note": PRECISION_NOTE[prec]}
+
+    if args.dump_outputs:
+        outputs = {k: sharding.gather_results(v, N) for k, v in outputs.items()}
+        if rank == 0:
+            write_outputs(Path(args.dump_outputs), outputs)
 
     # max over ranks
     times = torch.tensor([ms_total, ms_e2e, kernel_ms], dtype=torch.float64, device=dev)
@@ -528,7 +545,14 @@ def main():
     ap.add_argument("--chunk", type=int, default=50, help="Adam steps per kernel launch")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / gpu_eager_baseline legs")
     ap.add_argument("--no-other", action="store_true", help="skip the secondary arithmetic modes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed steps computed in their last step (energy, omega, adam_m, adam_v of "
+                         "every curve) as DIR/<name>.npy; the inputs are seeded, so two builds compare output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "vlg":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl vlg)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:
