@@ -19,7 +19,7 @@ out = (ctypes.c_longlong * (nc * 8))()
 lib.vlg_debug_tc_stats.argtypes = [ctypes.c_void_p, ctypes.c_int]
 assert lib.vlg_debug_tc_stats(out, nc) == 0
 st = np.array(out).reshape(nc, 8).astype(np.float64)
-names = ["-", "-", "mma wait full", "mma total", "epi0 wait acc", "mma issue loops", "epi1 wait acc", "-"]
+names = ["setup warp busy", "setup warp wait buffer", "mma wait full", "mma total", "epi0 wait acc", "mma issue loops", "epi1 wait acc", "-"]
 for i, nm in enumerate(names):
     if nm != "-":
         print(f"{nm:22s} mean {st[:, i].mean():12.0f} cycles  ({100 * st[:, i].mean() / st[:, 3].mean():5.1f}% of mma total)")
@@ -32,8 +32,8 @@ lib.vlg_debug_tc_phase.argtypes = [ctypes.c_void_p, ctypes.c_int]
 assert lib.vlg_debug_tc_phase(ph, nc) == 0
 ph = np.array(ph).reshape(nc, 2, 24).astype(np.float64).mean(0)
 names = ["F: item setup + sw wait", "F: layer 1 + st + arrive", "F: wait F2", "F: E-F2", "F: wait F3", "F: E-F3",
-         "window setup + row lists", "bar after forward", "energy pass", "B: setup + G build + arrive", "B: wait B3", "B: E-B3",
-         "B: wait B2", "B: E-B2 (dz)", "bar after backward", "domega + reductions", "step prologue/Adam", "w: points/draws", "w: count pass", "w: scan + item list", "e: loads + diff loop", "e: warp sum", "d: first barrier", "d: design rows + warp sums + bar"]
+         "window setup (points, wait lists)", "bar after forward", "energy pass", "B: setup + G build + arrive", "B: wait B3", "B: E-B3",
+         "B: wait B2", "B: E-B2 (dz)", "bar after backward", "domega + reductions", "step prologue/Adam", "-", "-", "-", "e: loads + diff loop", "e: warp sum", "d: first barrier", "d: design rows + warp sums + bar"]
 for c in range(2):
     tot = ph[c].sum()
     print(f"chain {c}: total {tot:.0f} cycles")

@@ -26,9 +26,9 @@ lib.vlg_debug_tc_phase.argtypes = [ctypes.c_void_p, ctypes.c_int]
 assert lib.vlg_debug_tc_phase(ph, nc) == 0
 ph = np.array(ph).reshape(nc, 2, 24).astype(np.float64).mean(0)
 names = ["F: item setup + sw wait", "F: layer 1 + st + arrive", "F: wait F2", "F: E-F2", "F: wait F3", "F: E-F3",
-         "window setup + row lists (place pass)", "bar after forward", "energy pass (+ tile pass)", "B: setup + G build + arrive", "B: wait B3", "B: E-B3",
+         "window setup (points, wait lists)", "bar after forward", "energy pass (+ tile pass)", "B: setup + G build + arrive", "B: wait B3", "B: E-B3",
          "B: wait B2", "B: E-B2 (dz)", "bar after backward", "domega + reductions", "step prologue/Adam",
-         "w: points/draws", "w: count pass", "w: scan + item list", "e: loads + diff loop", "e: warp sum", "d: first barrier", "d: design rows + warp sums + bar"]
+         "-", "-", "-", "e: loads + diff loop", "e: warp sum", "d: first barrier", "d: design rows + warp sums + bar"]
 for c in range(1):
     tot = ph[c].sum()
     print(f"chain {c}: total {tot:.0f} cycles per group-step (7 curves)")

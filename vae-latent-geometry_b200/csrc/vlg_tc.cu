@@ -1,6 +1,6 @@
 // tcgen05 geodesic step kernel -- the tensor-core variants.
 //
-// Persistent CTAs (one per SM, 608 threads) pull work units -- (curve, chunk of Adam steps) -- from
+// Persistent CTAs (one per SM, 640 threads) pull work units -- (curve, chunk of Adam steps) -- from
 // a global queue; a curve's chunks are chained through its omega/m/v in HBM, so a launch of
 // `steps` steps has no tail longer than one chunk.  The two 128-wide decoder layers and their
 // transposes run as tcgen05.mma with
@@ -27,14 +27,15 @@
 //
 // Warp roles: warps 0/1 = weight producers of chain 0/1 (one lane each), warp 2 = MMA issuer
 // (all lanes run the loop, one elected lane's instructions take effect), warps 3-10 and 11-18 = two
-// epilogue groups of 8 warps.  Each group owns a "chain"
+// epilogue groups of 8 warps, warp 19 = window setup.  Each group owns a "chain"
 // of 256 TMEM columns and every other item.  The MMA issuer serves whichever chain has its
 // operand ready, which is why every chain has its own weight ring.  Inside a group two threads
 // share a row (TMEM lane) and split its columns: four epilogue warps per scheduler hide TMEM /
 // shared-memory latency.
 //
-// Per window: draws (one word per point: the decoders of the <= 4 segment ends that meet there) ->
-// per-decoder row lists in point order (warp ballots + scans: deterministic item membership) ->
+// Per window, one window ahead in the setup warp: draws (one word per point: the decoders of the <= 4 segment ends
+// that meet there) -> per-decoder row lists in point order (deterministic item membership) -> item list; all of it
+// double buffered by window parity.  Then in the epilogue: points of the window ->
 // forward items (layer 1 on CUDA cores, exact fp32) -> selected outputs stored
 // with plain stores, one writer per slot (left-end output x1 of a segment in shared memory,
 // right-end output x2 in an L2-resident workspace) -> one pass forms x2-x1 and the energy ->
@@ -44,8 +45,8 @@
 // Where the time goes (VLG_TC_STATS build, per 128-row item of a chain, 3-term mode): 43 % epilogue phases
 // (7 per item, latency bound: two warps of a group per scheduler), 40 % waiting for the four GEMMs (a third of
 // it the MMAs themselves, the rest issue / commit / wake-up latency and the other chain's MMAs), 16 % per-window
-// phases (row lists, the x2-x1 pass: bandwidth of a 119 KB buffer, d(omega)).  Tensor memory holds two chains,
-// which is what bounds the overlap; see DESIGN.md 4.4 for the experiments that did not help.
+// phases (the x2-x1 pass: bandwidth of a 119 KB buffer, d(omega); in these round-2 figures also the row lists, which
+// the setup warp now builds off the chains).  Tensor memory holds two chains, which is what bounds the overlap; see DESIGN.md 4.4 for the experiments that did not help.
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
@@ -98,10 +99,11 @@ using namespace tc;
 #ifndef VLG_TC_G_AHEAD
 #define VLG_TC_G_AHEAD 1               // single-term backward: next item's dE/dx rows built under the current B2
 #endif
-constexpr int TC_THREADS = 608;       // 3 control warps + 16 epilogue warps
+constexpr int TC_THREADS = 640;       // 3 control warps + 16 epilogue warps + the window-setup warp
 constexpr int GROUP_THREADS = 256;    // one epilogue group (chain)
 constexpr int EPI_THREADS = 512;
 constexpr int FIRST_EPI_WARP = 3;
+constexpr int SETUP_WARP = FIRST_EPI_WARP + 16;
 constexpr int STAGE_BYTES = 16384;
 constexpr int MAX_STAGES = 5;         // per chain
 constexpr int XD_STRIDE = 52;         // floats per stored decoder output row (X <= 52; 16 B rows)
@@ -248,8 +250,9 @@ __host__ __device__ inline size_t tc_ws_cta_words(int K, int M, int W) {
 }
 
 struct WinCtl {
-  int nitems;
+  int nitems;    // < 0: no more work units
   int base;      // first decoder of the curve's weight set inside `packed` (StepParams::dec_base)
+  unsigned int unit;   // work unit the window belongs to (>= total units: no more work)
   uint16_t item[MAX_ITEMS];  // decoder | pass << 8
 };
 
@@ -262,13 +265,13 @@ __device__ __forceinline__ void acc_wait(uint64_t* bar, uint32_t parity, int lan
 struct TcSmem {
   unsigned char* ring;  // [chain][stage] 16 KB
   float* XD;            // [m][W][52] left-end outputs x1, then x2 - x1 (only when they fit: XL2 == 0; else in the workspace)
-  uint8_t* sel;         // [W + 1][4] per POINT: the decoders drawn for the segments that meet there -- byte 2m: left end of its own
-                        // segment (MC sample m), byte 2m+1: right end of the previous one; 255: none.  One 32-bit load per row.
-  uint16_t* rows;       // points of the window that drew decoder k, in increasing point order: rows[roff[k] .. + cnt[k])
-  uint16_t* wcnt;       // [K][chunks of 512 points][16 warps] rows per (decoder, chunk, warp) (then: exclusive prefix)
-  int* cnt;             // [K]
-  int* roff;            // [K]
-  WinCtl* ctl;          // [2] item lists, double buffered by window parity
+  // sel, rows, crow and ctl are written by the window-setup warp one window ahead: double buffered by window parity
+  uint8_t* sel;         // [2][tc_sel_words(W)][4] per POINT: the decoders drawn for the segments that meet there -- byte 2m: left
+                        // end of its own segment (MC sample m), byte 2m+1: right end of the previous one; 255: none (also every
+                        // byte of the words from W on).  One 32-bit load per row.
+  uint16_t* rows;       // [2][2 M W] points of the window that drew decoder k, in increasing point order: rows[roff[k] .. + cnt[k])
+  uint32_t* crow;       // [2][TC_MAX_K] roff[k] | cnt[k] << 16
+  WinCtl* ctl;          // [2] item lists
   float* sw;            // [chain][SW_SLOTS] 576 floats: W1 (planar), b1, b2, b3 of an item's decoder
   float2* zs;           // W latent points of the window
   float2* dzs;          // [4][W]: dz of point pt from the decoder of its draw slot (m0 left, m0 right, m1 left, m1 right)
@@ -280,13 +283,13 @@ struct TcSmem {
   float* etot;          // [G][2] energy / length of the step so far
   float* red;           // [16][20] d(omega) partials per warp, then [G][32] energy | length partials per warp
   float2* dzx;          // [chain][half][128] dz partial of a row's two half-threads (last backward item of the chain)
-  uint64_t* bars;       // full[2][MAX_STAGES], empty[2][MAX_STAGES], a_ready[2], acc_ready[2], win_ready, sw_full[2][SW_SLOTS], ctl_free[2], g_ready
-  uint32_t* tmem_base;  // [0] TMEM base address, [1] current work unit
+  uint64_t* bars;       // full[2][MAX_STAGES], empty[2][MAX_STAGES], a_ready[2], acc_ready[2], win_ready[2], sw_full[2][SW_SLOTS], ctl_free[2], g_ready
+  uint32_t* tmem_base;  // [0] TMEM base address
 };
 
 constexpr int CTL_FLOATS = (2 * sizeof(WinCtl) + 3) / 4;
 constexpr int SW_SLOTS = 4;            // small-weight buffers per chain (see the producer)
-constexpr int BAR_WORDS = 2 * (4 * MAX_STAGES + 5 + 2 * SW_SLOTS + 3);
+constexpr int BAR_WORDS = 2 * (4 * MAX_STAGES + 6 + 2 * SW_SLOTS + 3);
 static_assert(TC_MAX_M == 2, "the row-list build tests four candidates per point");
 
 // Fixed-size pieces first, at compile-time offsets from the start of dynamic shared memory (their
@@ -306,12 +309,13 @@ struct Fix {
   static constexpr int BARS = DZX + 1024;                         // BAR_WORDS (8-byte aligned)
   static constexpr int TMEM = BARS + BAR_WORDS;                  // 4
   static constexpr int CTL = TMEM + 4;                           // CTL_FLOATS
-  static constexpr int CNT = CTL + CTL_FLOATS;                   // TC_MAX_K
-  static constexpr int ROFF = CNT + TC_MAX_K;                    // TC_MAX_K
-  static constexpr int FLOATS = (ROFF + TC_MAX_K + 3) / 4 * 4;   // XD starts 16-byte aligned
+  static constexpr int CROW = CTL + CTL_FLOATS;                  // 2 x TC_MAX_K
+  static constexpr int FLOATS = (CROW + 2 * TC_MAX_K + 3) / 4 * 4;   // XD starts 16-byte aligned
 };
 
 __host__ __device__ inline int tc_chunks(int W) { return (W + 511) / 512; }
+// one buffer of TcSmem::sel: W + 1 words, rounded up to whole 16-byte loads
+__host__ __device__ inline int tc_sel_words(int W) { return (W + 1 + 3) / 4 * 4; }
 
 template <int GM>
 __device__ __forceinline__ TcSmem tc_carve(unsigned char* base, int W, int K, int M, bool xd_in_smem) {
@@ -330,16 +334,14 @@ __device__ __forceinline__ TcSmem tc_carve(unsigned char* base, int W, int K, in
   s.bars = reinterpret_cast<uint64_t*>(f + FX::BARS);
   s.tmem_base = reinterpret_cast<uint32_t*>(f + FX::TMEM);
   s.ctl = reinterpret_cast<WinCtl*>(f + FX::CTL);
-  s.cnt = reinterpret_cast<int*>(f + FX::CNT);
-  s.roff = reinterpret_cast<int*>(f + FX::ROFF);
+  s.crow = reinterpret_cast<uint32_t*>(f + FX::CROW);
   f += FX::FLOATS;
   s.XD = f; f += xd_in_smem ? M * W * XD_STRIDE : 0;
+  s.sel = reinterpret_cast<uint8_t*>(f); f += 2 * tc_sel_words(W);   // 16-byte aligned (read as uint4 by the setup warp)
   s.zs = reinterpret_cast<float2*>(f); f += 2 * W;
   s.dzs = reinterpret_cast<float2*>(f); f += 2 * 4 * W;
-  s.sel = reinterpret_cast<uint8_t*>(f); f += W + 1;
-  s.wcnt = reinterpret_cast<uint16_t*>(f); f += K * tc_chunks(W) * 8;
   s.rows = reinterpret_cast<uint16_t*>(f);
-  const size_t ring_off = (size_t(reinterpret_cast<unsigned char*>(f) - base) + size_t(2 * M) * W * 2 + 127) / 128 * 128;
+  const size_t ring_off = (size_t(reinterpret_cast<unsigned char*>(f) - base) + 2 * size_t(2 * M) * W * 2 + 127) / 128 * 128;
   s.ring = base + ring_off;
   return s;
 }
@@ -349,9 +351,8 @@ __device__ __forceinline__ TcSmem tc_carve(unsigned char* base, int W, int K, in
 static size_t tc_smem_fixed_bytes(int W, int K, int M, int xl2) {
   // everything but the weight rings, in the order of tc_carve (+ alignment slack before the rings)
   const size_t fix = xl2 ? Fix<TC_MAX_G>::FLOATS : Fix<1>::FLOATS;
-  size_t fl = fix + (xl2 ? 0 : size_t(M) * W * XD_STRIDE) + 2 * size_t(W) + 2 * 4 * size_t(W) + size_t(W) + 1 +
-              size_t(K) * tc_chunks(W) * 8;
-  return (fl * 4 + size_t(2 * M) * W * 2 + 127) / 128 * 128;
+  size_t fl = fix + (xl2 ? 0 : size_t(M) * W * XD_STRIDE) + 2 * size_t(tc_sel_words(W)) + 2 * size_t(W) + 2 * 4 * size_t(W);
+  return (fl * 4 + 2 * size_t(2 * M) * W * 2 + 127) / 128 * 128;
 }
 static int tc_stages(int W, int K, int M, int xl2) {
   const long budget = 232448 - long(tc_smem_fixed_bytes(W, K, M, xl2));
@@ -384,12 +385,14 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
   uint64_t* empty = s.bars + 2 * MAX_STAGES;     // [2][MAX_STAGES]
   uint64_t* a_ready = s.bars + 4 * MAX_STAGES;
   uint64_t* acc_ready = s.bars + 4 * MAX_STAGES + 2;
-  uint64_t* win_ready = s.bars + 4 * MAX_STAGES + 4;
-  uint64_t* sw_full = s.bars + 4 * MAX_STAGES + 5;   // [chain][SW_SLOTS]
-  // item list ctl[i] may be rewritten once both producers and both chain states of the issuer are done with it
-  uint64_t* ctl_free = s.bars + 4 * MAX_STAGES + 5 + 2 * SW_SLOTS;   // [2]
+  // window w's draws, row lists and item list are in buffer w & 1: win_ready[w & 1], phase w >> 1.  One barrier per
+  // buffer: a waiter is never two phases behind, because buffer b is rewritten only after ctl_free[b]
+  uint64_t* win_ready = s.bars + 4 * MAX_STAGES + 4;   // [2]
+  uint64_t* sw_full = s.bars + 4 * MAX_STAGES + 6;   // [chain][SW_SLOTS]
+  // buffer b may be rewritten once both producers, both chain states of the issuer and the epilogue are done with it
+  uint64_t* ctl_free = s.bars + 4 * MAX_STAGES + 6 + 2 * SW_SLOTS;   // [2]
   // the dE/dx operand tiles of the window are in the workspace (phase = window)
-  uint64_t* g_ready = s.bars + 4 * MAX_STAGES + 5 + 2 * SW_SLOTS + 2;
+  uint64_t* g_ready = s.bars + 4 * MAX_STAGES + 6 + 2 * SW_SLOTS + 2;
   const int nwin = (T - 1 + WSEG - 1) / WSEG;
   // work queue (zeroed by the host before the launch): [0] next unit, [64 + n] chunks done of curve n
   unsigned int* queue = reinterpret_cast<unsigned int*>(p.workspace);
@@ -407,10 +410,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
     mbar_init(&a_ready[1], GROUP_THREADS / 32);
     mbar_init(&acc_ready[0], 1);
     mbar_init(&acc_ready[1], 1);
-    mbar_init(win_ready, 1);
+    mbar_init(&win_ready[0], 1);
+    mbar_init(&win_ready[1], 1);
     for (int i = 0; i < 2 * SW_SLOTS; ++i) mbar_init(&sw_full[i], 1);
-    mbar_init(&ctl_free[0], 4);
-    mbar_init(&ctl_free[1], 4);
+    mbar_init(&ctl_free[0], 5);
+    mbar_init(&ctl_free[1], 5);
     mbar_init(g_ready, 1);
     fence_mbar_init();
   }
@@ -424,7 +428,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
   // Item i of a window (decoder k, rows 128q..128q+127 of k's row list) belongs to chain i & 1.
   // Per chain the tensor-core ops of a window are: for each of its items F2 F3, then (GRAD) for
   // each of its items B3 B2.  The item list of window w is published in ctl[w & 1] and
-  // announced through the win_ready mbarrier (phase = w).
+  // announced through win_ready[w & 1] (phase = w >> 1).
   if (warp < 2) {
     // ================= weight producer of chain `warp` (TMA bulk copies) =================
     if (lane == 0) {
@@ -440,7 +444,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
           reinterpret_cast<const uint32_t*>(p.workspace) + tc_queue_words(p.N) + size_t(blockIdx.x) * tc_ws_cta_words(K, M, W) +
           size_t(tc_max_items(K, M, W)) * 512 + 2 * size_t(M) * W * XD_STRIDE);
       for (long w = 0;; ++w) {
-        mbar_wait(win_ready, uint32_t(w & 1));
+        mbar_wait(&win_ready[w & 1], uint32_t((w >> 1) & 1));
         const WinCtl* ctl = &s.ctl[w & 1];
         const int nit = ctl->nitems;
         if (nit < 0) break;  // no more work units
@@ -527,7 +531,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
         for (int c = 0; c < 2; ++c) {
           if (fin[c]) continue;
           if (ops_left[c] == 0) {
-            if (!mbar_test(win_ready, uint32_t(win[c] & 1))) continue;
+            if (!mbar_test(&win_ready[win[c] & 1], uint32_t((win[c] >> 1) & 1))) continue;
             const int nit = s.ctl[win[c] & 1].nitems;
             if (nit < 0) { fin[c] = true; continue; }
             mbar_arrive_elect(&ctl_free[win[c] & 1], leader);   // the issuer only needs the item count
@@ -636,7 +640,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
 #endif
       (void)w_full; (void)w_issue;
     }
-  } else {
+  } else if (warp < SETUP_WARP) {
     // ================= epilogue groups =================
     const int ew = warp - FIRST_EPI_WARP;       // 0..15
     const int chain_id = ew >> 3;               // group / chain
@@ -657,8 +661,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
     const float coefm = 2.0f / float(Mtot);
     long long w_acc = 0;
     long wcount = 0;                            // windows processed by this CTA so far
-    bool bad_draw = false;                      // an explicit draw was >= K (clamped)
-    unsigned long long n_items = 0, n_rows = 0; // executed 128-row items / occupied rows (thread 0; launch statistics)
     // this CTA's slice of the L2-resident workspace (tc_ws_cta_words): ReLU masks, both end-point outputs of
     // every segment, and the dE/dx operand tiles one fused pass builds from them for the backward items
     uint32_t* maskws = reinterpret_cast<uint32_t*>(p.workspace) + tc_queue_words(p.N) + size_t(blockIdx.x) * tc_ws_cta_words(K, M, W);
@@ -673,23 +675,21 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
 
     for (;;) {
       // ---- next work unit: (group of G curves n0 .. n0 + Gcur - 1, steps [step_lo, step_hi)) ----
-      if (t512 == 0) {
-        const unsigned int u = atomicAdd(&queue[0], 1u);
-        s.tmem_base[1] = u;
-        if (u < total_units && u >= ngroups) {
-          // a later chunk of a group: wait until its previous chunk has been written back
-          const unsigned int* flag = &queue[64 + u % ngroups];
-          const unsigned int need = u / ngroups;
-          unsigned int have;
-          do {
-            asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(have) : "l"(flag) : "memory");
-            if (have < need) __nanosleep(100);
-          } while (have < need);
-        }
+      // The setup warp pulls it from the queue and names it in the item list of the unit's first window.
+      mbar_wait(&win_ready[wcount & 1], uint32_t((wcount >> 1) & 1));
+      const unsigned int unit = s.ctl[wcount & 1].unit;
+      if (unit >= total_units) break;
+      if (t512 == 0 && unit >= ngroups) {
+        // a later chunk of a group: wait until its previous chunk has been written back
+        const unsigned int* flag = &queue[64 + unit % ngroups];
+        const unsigned int need = unit / ngroups;
+        unsigned int have;
+        do {
+          asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(have) : "l"(flag) : "memory");
+          if (have < need) __nanosleep(100);
+        } while (have < need);
       }
       named_bar(3, EPI_THREADS);
-      const unsigned int unit = s.tmem_base[1];
-      if (unit >= total_units) break;
       const int grp = int(unit % ngroups);
       const int n0 = grp * G, Gcur = XL2 ? min(G, p.N - n0) : 1;
       const int chunk = int(unit / ngroups);
@@ -710,12 +710,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
       if (t512 < 4 * G) {
         const int j = t512 >> 2, c = t512 & 3, n = n0 + min(j, Gcur - 1);
         s.pab[t512] = c < 2 ? p.a[2 * n + c] : p.b[2 * n + c - 2];
-      }
-      // one weight set per window: per-curve sets (decoder_base) are only launched with G = 1
-      int dec_base = p.dec_base ? p.dec_base[n0] : 0;
-      if (dec_base < 0 || dec_base + K > p.K_total) {   // memory safety; reported through the status word
-        dec_base = 0;
-        if (t512 == 0) atomicOr(&queue[1], unsigned(VLG_STATUS_BAD_PACKED));
       }
       named_bar(3, EPI_THREADS);
 
@@ -738,141 +732,32 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
           const int Mb = min(TC_MAX_M, Mtot - 2 * mb);   // samples of this block
           const int seg0 = win * WSEG;
           const int nseg = min(WSEG, T - 1 - seg0);   // segments of every curve in this window
-          WinCtl* ctl = &s.ctl[wcount & 1];
-          // ---- window setup: points, draws, accumulators (point pt = curve j = pt / Wp, local index i) ----
-          for (int pt = t512; pt < W; pt += EPI_THREADS) {
+          // ---- window setup: draws, row lists and item list from the setup warp; points and dz accumulators here ----
+          const int buf = int(wcount & 1);
+          mbar_wait(&win_ready[buf], uint32_t((wcount >> 1) & 1));
+          const WinCtl* ctl = &s.ctl[buf];
+          const uint8_t* sel = s.sel + size_t(buf) * tc_sel_words(W) * 4;
+          const uint16_t* rows = s.rows + size_t(buf) * 2 * M * W;
+          const uint32_t* crow = s.crow + buf * TC_MAX_K;
+          for (int pt = t512; pt < W; pt += EPI_THREADS) {   // point pt = curve j = pt / Wp, local index i
             const int j = pt / Wp, i = pt - j * Wp;
-            const int ti = min(seg0 + i, T - 1);
             const float* ab = s.pab + 4 * j;
-            s.zs[pt] = spline_point(p.t[ti], n_poly, s.coef + j * 64, make_float2(ab[0], ab[1]), make_float2(ab[2], ab[3]));
-            const bool seg_ok = i < nseg && j < Gcur;
-            const int n = n0 + j;
-            if (p.draws != nullptr) {
-              for (int m = 0; m < Mb; ++m)
-                for (int role = 0; role < 2; ++role) {
-                  uint8_t v = 255;
-                  if (seg_ok) {
-                    v = p.draws[(((size_t(n) * p.steps + step) * Mtot + 2 * mb + m) * 2 + role) * size_t(T - 1) + seg0 + i];
-                    if (v >= K) { v = uint8_t(K - 1); bad_draw = true; }   // memory safety; reported through the status word
-                  }
-                  s.sel[4 * (pt + role) + 2 * m + role] = v;
-                }
-              if (Mb < 2) { s.sel[4 * pt + 2] = 255; s.sel[4 * pt + 7] = 255; }
-            } else {
-              uint32_t d[4] = {255u, 255u, 255u, 255u};
-              if (seg_ok)
-                counter_draws4(p.seed, uint32_t(p.curve_id0 + n), uint32_t(p.step0 + step), uint32_t(seg0 + i), uint32_t(mb),
-                               uint32_t(K), d);
-              for (int q = 0; q < 4; ++q) s.sel[4 * (pt + (q & 1)) + q] = (q >> 1) < Mb ? uint8_t(d[q]) : uint8_t(255);
-            }
-            if (pt == 0) { s.sel[1] = 255; s.sel[3] = 255; }   // no segment ends at the first point
+            s.zs[pt] = spline_point(p.t[min(seg0 + i, T - 1)], n_poly, s.coef + j * 64, make_float2(ab[0], ab[1]),
+                                    make_float2(ab[2], ab[3]));
           }
           for (int i = t512; i < 4 * W; i += EPI_THREADS) s.dzs[i] = make_float2(0.f, 0.f);
-          named_bar(3, EPI_THREADS);
-          PHW(17);
-          // ---- per-decoder row lists, in increasing point order ----
-          // Item membership must not depend on thread timing: a decoder drawn by more than 128 points of
-          // the window is split into several items, which run on different chains, and the chains' dz
-          // partial sums are added in a fixed order -- so WHICH points share an item fixes the fp32
-          // summation grouping.  Ordered compaction: thread = point (chunks of 512 points), each warp owns
-          // 32 consecutive points; per decoder a ballot gives the rank inside the warp, a scan over
-          // (chunk, warp) the warp's base, a scan over the decoders each list's offset.  Two passes over
-          // the ballots: count, then place.  (Bit-identical results for any sharding / scheduling.)
-          const uint32_t lt = (1u << lane) - 1u;
-          const int wpos = t512 >> 5;                 // position of this warp's 32 points inside a chunk
-          auto candidates = [&](int pt, int (&cand)[2 * TC_MAX_M]) {
-#pragma unroll
-            for (int i = 0; i < 2 * TC_MAX_M; ++i) cand[i] = -1;
-            if (pt < W) {
-              const uint32_t c4 = reinterpret_cast<const uint32_t*>(s.sel)[pt];
-#pragma unroll
-              for (int i = 0; i < 2 * TC_MAX_M; ++i) {
-                const int c = int((c4 >> (8 * i)) & 0xFFu);
-                if (c != 255) cand[i] = c;
-              }
-#pragma unroll
-              for (int i = 1; i < 2 * TC_MAX_M; ++i)
-#pragma unroll
-                for (int j = 0; j < i; ++j)
-                  if (cand[j] == cand[i]) cand[i] = -1;   // a point enters a decoder's list once
-            }
-          };
-          for (int ch = 0; ch < nchunk; ++ch) {
-            int cand[2 * TC_MAX_M];
-            candidates(ch * 512 + t512, cand);
-            for (int k = 0; k < K; ++k) {
-              const bool mem = (cand[0] == k) | (cand[1] == k) | (cand[2] == k) | (cand[3] == k);
-              const uint32_t bal = __ballot_sync(0xffffffffu, mem);
-              if (lane == 0) s.wcnt[(k * nchunk + ch) * 16 + wpos] = uint16_t(__popc(bal));
-            }
-          }
-          named_bar(3, EPI_THREADS);
-          PHW(18);
-          if (t512 < 32) {
-            // One warp, lane = decoder (32 at a time): the scan over (chunk, warp) per decoder, then warp scans over the
-            // decoders for the list offsets and the item numbers; every lane writes its decoder's items.
-            // The control warps must be done with the item list this one replaces (window wcount - 2).
-            if (lane == 0 && wcount >= 2) mbar_wait(&ctl_free[wcount & 1], uint32_t(((wcount >> 1) - 1) & 1));
-            __syncwarp();
-            int off_carry = 0, ni_carry = 0;
-            for (int k0 = 0; k0 < K; k0 += 32) {
-              const int k = k0 + lane;
-              int acc = 0;
-              if (k < K)
-                for (int w = 0; w < nchunk * 16; ++w) {
-                  const int c = s.wcnt[k * nchunk * 16 + w];
-                  s.wcnt[k * nchunk * 16 + w] = uint16_t(acc);
-                  acc += c;
-                }
-              const int nit = (acc + 127) >> 7;
-              int so = acc, si = nit;   // inclusive scans over the lanes
-#pragma unroll
-              for (int o = 1; o < 32; o <<= 1) {
-                const int a = __shfl_up_sync(0xffffffffu, so, o), b = __shfl_up_sync(0xffffffffu, si, o);
-                if (lane >= o) { so += a; si += b; }
-              }
-              if (k < K) {
-                s.cnt[k] = acc;
-                s.roff[k] = off_carry + so - acc;
-                const int i0 = ni_carry + si - nit;
-                for (int q = 0; q < nit; ++q) ctl->item[i0 + q] = uint16_t(k | (q << 8));
-              }
-              off_carry += __shfl_sync(0xffffffffu, so, 31);
-              ni_carry += __shfl_sync(0xffffffffu, si, 31);
-            }
-            if (lane == 0) {
-              ctl->nitems = ni_carry;
-              ctl->base = dec_base;
-              n_items += unsigned(ni_carry);
-              n_rows += unsigned(off_carry);
-            }
-            __threadfence_block();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(win_ready);
-          }
-          named_bar(3, EPI_THREADS);
-          PHW(19);
-          for (int ch = 0; ch < nchunk; ++ch) {
-            int cand[2 * TC_MAX_M];
-            const int pt = ch * 512 + t512;
-            candidates(pt, cand);
-            for (int k = 0; k < K; ++k) {
-              const bool mem = (cand[0] == k) | (cand[1] == k) | (cand[2] == k) | (cand[3] == k);
-              const uint32_t bal = __ballot_sync(0xffffffffu, mem);
-              if (mem) s.rows[s.roff[k] + s.wcnt[(k * nchunk + ch) * 16 + wpos] + __popc(bal & lt)] = uint16_t(pt);
-            }
-          }
           named_bar(3, EPI_THREADS);
           const int nitems = ctl->nitems;
           PH(6);
           // =============================== forward ===============================
           for (int it = chain_id; it < nitems; it += 2) {
             const int k = ctl->item[it] & 0xFF, q0 = (ctl->item[it] >> 8) * 128;
-            const bool active = q0 + row < s.cnt[k];
+            const uint32_t cr = crow[k];
+            const bool active = q0 + row < int(cr >> 16);
             // tcgen05.ld/st are warp-collective (.sync.aligned): a warp takes part as soon as one of
             // its 32 rows is in use; unused lanes compute on point 0 and store nothing
-            const bool wact = q0 + (warp & 3) * 32 < s.cnt[k];
-            const int pt = active ? s.rows[s.roff[k] + q0 + row] : 0;
+            const bool wact = q0 + (warp & 3) * 32 < int(cr >> 16);
+            const int pt = active ? rows[(cr & 0xFFFFu) + q0 + row] : 0;
             // small weights of decoder k: loaded by the chain's producer (bulk copy -> mbarrier).  TF32
             // operands overwrite accumulators in place, so the group must also be done with the previous
             // item's D3 before layer 1 is stored; fp16 operands and accumulators never share columns.
@@ -1013,7 +898,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
               }
               // the slots of this point that drew decoder k (one compare for all four).  Even slot 2m: this point is the left
               // end of its segment (-> x1 row of the segment); odd slot 2m+1: right end of the previous one (-> x2 row)
-              const uint32_t eq = active ? slot_match(s.sel, pt, k) : 0u;
+              const uint32_t eq = active ? slot_match(sel, pt, k) : 0u;
 #pragma unroll
               for (int j = 0; j < 2 * TC_MAX_M; ++j)
                 if (eq & (1u << (8 * j))) {
@@ -1126,11 +1011,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
                 if (t0 < ntask) {
                   const int it = t0 >> 10, r = (t0 >> 3) & 127, c = t0 & 7;
                   const int k = ctl->item[it] & 0xFF, q0 = (ctl->item[it] >> 8) * 128;
-                  if (q0 + r < s.cnt[k]) {
-                    const int pt = s.rows[s.roff[k] + q0 + r];
+                  const uint32_t cr = crow[k];
+                  if (q0 + r < int(cr >> 16)) {
+                    const int pt = rows[(cr & 0xFFFFu) + q0 + r];
                     ptv[u] = pt;
                     if (c < 7) {   // chunk 7 = zero padding (columns 56..63)
-                      const uint32_t eq4 = slot_match(s.sel, pt, k);
+                      const uint32_t eq4 = slot_match(sel, pt, k);
                       // bit j: slot j in the order right end of segment pt-1 (sample 0), left end of segment pt (sample 0), ...
                       const uint32_t mk = ((eq4 >> 8) & 1u) | ((eq4 << 1) & 2u) | ((eq4 >> 22) & 4u) | ((eq4 >> 13) & 8u);
                       mkv[u] = mk;
@@ -1260,7 +1146,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
                   float g[32];
   #pragma unroll
                   for (int j = 0; j < 32; ++j) g[j] = 0.f;
-                  const uint32_t eq = active ? slot_match(s.sel, pt, k) : 0u;
+                  const uint32_t eq = active ? slot_match(sel, pt, k) : 0u;
 #pragma unroll
                   for (int m = 0; m < TC_MAX_M; ++m) {     // same order of additions as ever: right end, then left end, per sample
                     if (eq & (0x100u << (16 * m))) {
@@ -1307,9 +1193,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
             auto item_row = [&](int it2, int& k2, int& pt2, bool& act2, bool& wact2) {
               k2 = ctl->item[it2] & 0xFF;
               const int q02 = (ctl->item[it2] >> 8) * 128;
-              act2 = q02 + row < s.cnt[k2];
-              wact2 = q02 + (warp & 3) * 32 < s.cnt[k2];
-              pt2 = act2 ? s.rows[s.roff[k2] + q02 + row] : 0;
+              const uint32_t cr2 = crow[k2];
+              act2 = q02 + row < int(cr2 >> 16);
+              wact2 = q02 + (warp & 3) * 32 < int(cr2 >> 16);
+              pt2 = act2 ? rows[(cr2 & 0xFFFFu) + q02 + row] : 0;
             };
             if (G_AHEAD && chain_id < nitems) {   // the first item of the chain
               int k2, pt2; bool a2, w2;
@@ -1321,9 +1208,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
             }
             for (int it = chain_id; it < nitems; it += 2) {
               const int k = ctl->item[it] & 0xFF, q0 = (ctl->item[it] >> 8) * 128;
-              const bool active = q0 + row < s.cnt[k];
-              const bool wact = q0 + (warp & 3) * 32 < s.cnt[k];
-              const int pt = active ? s.rows[s.roff[k] + q0 + row] : 0;
+              const uint32_t cr = crow[k];
+              const bool active = q0 + row < int(cr >> 16);
+              const bool wact = q0 + (warp & 3) * 32 < int(cr >> 16);
+              const int pt = active ? rows[(cr & 0xFFFFu) + q0 + row] : 0;
               mbar_wait(&sw_full[chain_id * SW_SLOTS + (swj % SW_SLOTS)], (swj / SW_SLOTS) & 1u);
               if (!F16) named_bar(bar_id, GROUP_THREADS);
               const float* sw = swbuf + (swj % SW_SLOTS) * 576;
@@ -1438,7 +1326,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
               pend_pt = -1;
               if (active && half == 0) {
                 pend_pt = pt;
-                pend_slot = (__ffs(int(slot_match(s.sel, pt, k))) - 1) >> 3;   // first draw slot of the point that holds decoder k
+                pend_slot = (__ffs(int(slot_match(sel, pt, k))) - 1) >> 3;   // first draw slot of the point that holds decoder k
               }
               PH(13);
               if (G_AHEAD && it + 2 < nitems) {   // D5 is in registers (tcgen05.wait::ld): B3 of the next item may overwrite Y
@@ -1454,6 +1342,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
             }
           }
           named_bar(3, EPI_THREADS);
+          if (t512 == 0) mbar_arrive(&ctl_free[buf]);   // done with this window's draws and lists: the buffer may be rewritten
           PHW(22);
           // ---- energy of the window per curve; d(omega) += P^T dz over the points of the window ----
           if (t512 < Gcur) {
@@ -1551,23 +1440,171 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
         asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(&queue[64 + grp]), "r"(v) : "memory");
       }
     }  // work units
-    if (bad_draw) atomicOr(&queue[1], unsigned(VLG_STATUS_BAD_DRAW));
-    if (t512 == 0) {   // launch statistics for vlg_workspace_counters (words [2..5] of the header)
-      atomicAdd(reinterpret_cast<unsigned long long*>(queue + 2), n_items);
-      atomicAdd(reinterpret_cast<unsigned long long*>(queue + 4), n_rows);
-    }
-    // tell the control warps that there is no more work
-    if (t512 == 0) {
-      if (wcount >= 2) mbar_wait(&ctl_free[wcount & 1], uint32_t(((wcount >> 1) - 1) & 1));
-      s.ctl[wcount & 1].nitems = -1;
-      __threadfence_block();
-      mbar_arrive(win_ready);
-    }
 #ifdef VLG_TC_STATS
     if (tg == 0 && blockIdx.x < 1024) g_tc_stats[blockIdx.x * 8 + 4 + chain_id * 2] = w_acc;
 #endif
     PH_FLUSH();
     (void)w_acc;
+  } else {
+    // ================= window setup: draws, row lists and item lists, one window ahead of the epilogue =================
+    // Runs through the same (work unit, step, window, sample block) sequence as the epilogue.  Nothing here depends on
+    // a window's results: the draws are counter-based (or read from p.draws), the lists depend on the draws only.
+    // Window w is built into buffer w & 1 once every consumer -- producers, issuer, epilogue -- is done with window
+    // w - 2 (ctl_free), and announced on win_ready[w & 1].
+    long wseq = 0;                              // windows set up so far
+    bool bad_draw = false;                      // an explicit draw was >= K (clamped)
+    unsigned long long n_items = 0, n_rows = 0; // 128-row items / occupied rows (launch statistics)
+    const int selw = tc_sel_words(W);
+#ifdef VLG_TC_STATS
+    long long t_busy = 0, t_free = 0;
+#endif
+    auto claim_buffer = [&]() {
+#ifdef VLG_TC_STATS
+      const long long t0 = clock64();
+#endif
+      if (wseq >= 2) mbar_wait(&ctl_free[wseq & 1], uint32_t(((wseq >> 1) - 1) & 1));
+#ifdef VLG_TC_STATS
+      t_free += clock64() - t0;
+#endif
+    };
+    unsigned int unit;
+    for (;;) {
+      claim_buffer();
+      unit = 0;
+      if (lane == 0) unit = atomicAdd(&queue[0], 1u);
+      unit = __shfl_sync(0xffffffffu, unit, 0);
+      if (unit >= total_units) break;
+      const int grp = int(unit % ngroups);
+      const int n0 = grp * G, Gcur = XL2 ? min(G, p.N - n0) : 1;
+      const int chunk = int(unit / ngroups);
+      const int step_lo = chunk * unit_steps, step_hi = min(p.steps, step_lo + unit_steps);
+      // one weight set per window: per-curve sets (decoder_base) are only launched with G = 1
+      int dec_base = p.dec_base ? p.dec_base[n0] : 0;
+      if (dec_base < 0 || dec_base + K > p.K_total) {   // memory safety; reported through the status word
+        dec_base = 0;
+        if (lane == 0) atomicOr(&queue[1], unsigned(VLG_STATUS_BAD_PACKED));
+      }
+      for (int step = step_lo; step < step_hi; ++step)
+        for (int win = 0; win < nwin; ++win)
+          for (int mb = 0; 2 * mb < Mtot; ++mb, ++wseq) {
+            const int Mb = min(TC_MAX_M, Mtot - 2 * mb);   // samples of this block
+            const int seg0 = win * WSEG;
+            const int nseg = min(WSEG, T - 1 - seg0);     // segments of every curve in this window
+            const int buf = int(wseq & 1);
+            claim_buffer();
+#ifdef VLG_TC_STATS
+            const long long t0 = clock64();
+#endif
+            uint8_t* sel = s.sel + size_t(buf) * selw * 4;
+            uint16_t* rows = s.rows + size_t(buf) * 2 * M * W;
+            uint32_t* crow = s.crow + buf * TC_MAX_K;
+            WinCtl* ctl = &s.ctl[buf];
+            // ---- draws: one word per point (lane = point).  Words W .. selw-1 hold no draw (255) ----
+            for (int i = W + lane; i < selw; i += 32) reinterpret_cast<uint32_t*>(sel)[i] = 0xFFFFFFFFu;
+            __syncwarp();
+            for (int pt = lane; pt < W; pt += 32) {
+              const int j = pt / Wp, i = pt - j * Wp;   // point pt = curve j = pt / Wp, local index i
+              const bool seg_ok = i < nseg && j < Gcur;
+              const int n = n0 + j;
+              if (p.draws != nullptr) {
+                for (int m = 0; m < Mb; ++m)
+                  for (int role = 0; role < 2; ++role) {
+                    uint8_t v = 255;
+                    if (seg_ok) {
+                      v = p.draws[(((size_t(n) * p.steps + step) * Mtot + 2 * mb + m) * 2 + role) * size_t(T - 1) + seg0 + i];
+                      if (v >= K) { v = uint8_t(K - 1); bad_draw = true; }   // memory safety; reported through the status word
+                    }
+                    sel[4 * (pt + role) + 2 * m + role] = v;
+                  }
+                if (Mb < 2) { sel[4 * pt + 2] = 255; sel[4 * pt + 7] = 255; }
+              } else {
+                uint32_t d[4] = {255u, 255u, 255u, 255u};
+                if (seg_ok)
+                  counter_draws4(p.seed, uint32_t(p.curve_id0 + n), uint32_t(p.step0 + step), uint32_t(seg0 + i), uint32_t(mb),
+                                 uint32_t(K), d);
+                for (int q = 0; q < 4; ++q) sel[4 * (pt + (q & 1)) + q] = (q >> 1) < Mb ? uint8_t(d[q]) : uint8_t(255);
+              }
+              if (pt == 0) { sel[1] = 255; sel[3] = 255; }   // no segment ends at the first point
+            }
+            __syncwarp();
+            // ---- per-decoder row lists, in increasing point order ----
+            // Item membership must not depend on thread timing: a decoder drawn by more than 128 points of the
+            // window is split into several items, which run on different chains, and the chains' dz partial sums
+            // are added in a fixed order -- so WHICH points share an item fixes the fp32 summation grouping.
+            // Lane = decoder (32 at a time): a count pass over the points, scans over the lanes for the list
+            // offsets and item numbers, then a pass that appends every matching point to the lane's own list.
+            // A point enters a decoder's list once, whichever of its draw slots hold the decoder.
+            const uint4* sel4 = reinterpret_cast<const uint4*>(sel);
+            auto holds = [](uint32_t w, uint32_t kp) {   // some byte of w equals the byte of kp (exact zero-byte test)
+              const uint32_t y = w ^ kp;
+              return ((y - 0x01010101u) & ~y & 0x80808080u) != 0u;
+            };
+            int off_carry = 0, ni_carry = 0;
+            for (int k0 = 0; k0 < K; k0 += 32) {
+              const int k = k0 + lane;   // k >= K matches no byte: draws are < K or 255
+              const uint32_t kp = uint32_t(k) * 0x01010101u;
+              int cnt = 0;
+              for (int q = 0; 4 * q < W; ++q) {
+                const uint4 v = sel4[q];
+                cnt += int(holds(v.x, kp)) + int(holds(v.y, kp)) + int(holds(v.z, kp)) + int(holds(v.w, kp));
+              }
+              const int nit = (cnt + 127) >> 7;
+              int so = cnt, si = nit;   // inclusive scans over the lanes
+#pragma unroll
+              for (int o = 1; o < 32; o <<= 1) {
+                const int a = __shfl_up_sync(0xffffffffu, so, o), b = __shfl_up_sync(0xffffffffu, si, o);
+                if (lane >= o) { so += a; si += b; }
+              }
+              const int roff = off_carry + so - cnt;
+              if (k < K) {
+                crow[k] = uint32_t(roff) | (uint32_t(cnt) << 16);
+                const int i0 = ni_carry + si - nit;
+                for (int q = 0; q < nit; ++q) ctl->item[i0 + q] = uint16_t(k | (q << 8));
+              }
+              off_carry += __shfl_sync(0xffffffffu, so, 31);
+              ni_carry += __shfl_sync(0xffffffffu, si, 31);
+              uint16_t* out = rows + roff;
+              for (int q = 0; 4 * q < W; ++q) {
+                const uint4 v = sel4[q];
+                if (holds(v.x, kp)) *out++ = uint16_t(4 * q);
+                if (holds(v.y, kp)) *out++ = uint16_t(4 * q + 1);
+                if (holds(v.z, kp)) *out++ = uint16_t(4 * q + 2);
+                if (holds(v.w, kp)) *out++ = uint16_t(4 * q + 3);
+              }
+            }
+            if (lane == 0) {
+              ctl->nitems = ni_carry;
+              ctl->base = dec_base;
+              ctl->unit = unit;
+              n_items += unsigned(ni_carry);
+              n_rows += unsigned(off_carry);
+            }
+            __threadfence_block();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&win_ready[buf]);
+#ifdef VLG_TC_STATS
+            t_busy += clock64() - t0;
+#endif
+          }
+    }
+    // no more work: an item list with no items, in the buffer of the next window
+    if (lane == 0) {
+      s.ctl[wseq & 1].nitems = -1;
+      s.ctl[wseq & 1].unit = unit;
+      __threadfence_block();
+      mbar_arrive(&win_ready[wseq & 1]);
+    }
+    if (bad_draw) atomicOr(&queue[1], unsigned(VLG_STATUS_BAD_DRAW));
+    if (lane == 0) {   // launch statistics for vlg_workspace_counters (words [2..5] of the header)
+      atomicAdd(reinterpret_cast<unsigned long long*>(queue + 2), n_items);
+      atomicAdd(reinterpret_cast<unsigned long long*>(queue + 4), n_rows);
+    }
+#ifdef VLG_TC_STATS
+    if (lane == 0 && blockIdx.x < 1024) {
+      g_tc_stats[blockIdx.x * 8 + 0] = t_busy;
+      g_tc_stats[blockIdx.x * 8 + 1] = t_free;
+    }
+#endif
   }
 
   tc_fence_before();
