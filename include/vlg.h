@@ -52,8 +52,9 @@ enum {
 enum {
   VLG_STATUS_BAD_DRAW = 1,  /* an explicit draw was >= K_active (the kernel clamped it to K_active-1) */
   VLG_STATUS_BAD_PACKED = 4, /* `packed` does not start with a header of the K / X the caller passed */
-  VLG_STATUS_NONFINITE = 2  /* an energy or an updated omega was inf/NaN: with VLG_PRECISION_F16* this is
-                               what an operand beyond the fp16 range (65504) turns into              */
+  VLG_STATUS_NONFINITE = 2  /* an energy, an updated omega or (vlg_curve_energy_grad) a gradient component was
+                               inf/NaN: with VLG_PRECISION_F16* this is what an operand beyond the fp16 range
+                               (65504) turns into                                                      */
 };
 
 /* Arithmetic used for the two 128-wide decoder layers (and their transposes). */
@@ -129,7 +130,7 @@ int vlg_optimize_steps(const void* packed, int K, int X, int K_active, int N, in
                        float* energy_last, float* energy_trace, int precision,
                        void* workspace, size_t workspace_bytes, void* stream);
 
-/* Status of the last vlg_optimize_steps / vlg_curve_energy launch that used `workspace`: copies the
+/* Status of the last vlg_optimize_steps / vlg_curve_energy / vlg_curve_energy_grad launch that used `workspace`: copies the
  * status word back and SYNCHRONISES `stream` (the only entry point that does).  *flags (host
  * pointer, may be NULL) receives the VLG_STATUS_* bits; returns VLG_OK when none is set, else
  * VLG_ERR_NUMERIC.  Replaces the finite-check a caller of the reference would do on `energy`
@@ -158,6 +159,25 @@ int vlg_curve_energy(const void* packed, int K, int X, int K_active, int N, int 
                      int step, float* energy, float* length, int precision, void* workspace,
                      size_t workspace_bytes, void* stream);
 
+/* ---- differentiable energy --------------------------------------------------------------
+ * Replaces the autograd backward of the energy at src/optimize.py:161 (`loss.sum().backward()`, the energy's
+ * part of it): ONE launch of the optimiser's step kernel that evaluates energy[N] exactly as vlg_curve_energy
+ * (same arguments, same draw stream at `step`) and its gradient with respect to the curve parameters
+ *   grad_omega [N,Kb,2] = dE/d(omega) = sum_t P[t]^T dz[t]
+ *   grad_a     [N,2]    = dE/da      = sum_t (1-t) dz[t]
+ *   grad_b     [N,2]    = dE/db      = sum_t t dz[t]
+ * where dz[t] = dE/dz[t] flows back through the decoders (decoder weight gradients are not formed).  The energy
+ * alone: no end-point penalty term (the reference's compute_energy_mc has none), no Adam, omega is not written.
+ * The energy is bit-identical to the first step of vlg_optimize_steps with the same inputs; grad_omega is the
+ * gradient that step hands to Adam minus its penalty term.  All output pointers are required; the workspace is
+ * vlg_workspace_bytes as for the other step-kernel calls and vlg_workspace_status reads its status.
+ */
+int vlg_curve_energy_grad(const void* packed, int K, int X, int K_active, int N, int T, int n_poly, int M,
+                          const float* a, const float* b, const float* omega, const float* basis,
+                          const float* t, const uint8_t* draws, const int32_t* decoder_base, uint64_t seed,
+                          int64_t curve_id0, int step, float* energy, float* grad_omega, float* grad_a,
+                          float* grad_b, int precision, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- ensemble disagreement field ------------------------------------------------------
  * out[g] = || std_k f_k(grid[g]) ||_2 over the first K_active decoders, unbiased std
  * (src/init_splines_ensemble.py:49-51, before the min-max normalisation).  grid [G,2].
@@ -172,6 +192,15 @@ int vlg_ensemble_std_norm(const void* packed, int K, int X, int K_active, int G,
 int vlg_spline_points(int N, int T, int n_poly, const float* a, const float* b,
                       const float* omega, const float* basis, const float* t, float* z,
                       void* stream);
+
+/* Backward of vlg_spline_points: the spline's part of the autograd backward at src/optimize.py:161 (the
+ * end-point penalty `model(torch.tensor([1.0]))`, 158-160, or any loss on z).  For dz[T,N,2] = dL/dz:
+ *   grad_omega[N,Kb,2] = sum_t P[t]^T dz[t],  grad_a[N,2] = sum_t (1-t) dz[t],  grad_b[N,2] = sum_t t dz[t].
+ * Fixed summation order, no atomics: repeated calls give the same bits.
+ */
+int vlg_spline_points_backward(int N, int T, int n_poly, const float* basis, const float* t,
+                               const float* dz, float* grad_omega, float* grad_a, float* grad_b,
+                               void* stream);
 
 /* ---- spline fit to a poly-line ----------------------------------------------------------
  * omega[n] = argmin mean((lin + P_L omega - target_n)^2), the optimum that the reference's

@@ -34,8 +34,14 @@ SIGNATURES = {
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                  c_uint64, c_int64, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                  c_size_t, c_void_p]),
+    "vlg_curve_energy_grad": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_uint64, c_int64, c_int,                      # seed id0 step
+                                      c_void_p, c_void_p, c_void_p, c_void_p,         # energy grad_omega grad_a grad_b
+                                      c_int, c_void_p, c_size_t, c_void_p]),
     "vlg_ensemble_std_norm": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "vlg_spline_points": (c_int, [c_int, c_int, c_int] + [c_void_p] * 7),
+    "vlg_spline_points_backward": (c_int, [c_int, c_int, c_int] + [c_void_p] * 7),
     "vlg_fit_splines": (c_int, [c_int, c_int, c_int] + [c_void_p] * 6),
 }
 

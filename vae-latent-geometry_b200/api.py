@@ -7,6 +7,8 @@ Same names and argument meaning as the reference where a counterpart exists:
   list(model.decoder)            (src/optimize.py:103)  DecoderEnsemble.from_state_dict(...)
   GeodesicSplineBatch(a,b,basis,omega,n_poly)   (13-35)  GeodesicSplineBatch (same signature)
   compute_energy_mc(model, decoders, t_vals, M) (38-75)  compute_energy_mc (same signature, +draws/seed)
+  loss.sum().backward()                           (161)  autograd through compute_energy_mc and
+                                                           GeodesicSplineBatch.forward (omega, a, b)
   optim.Adam([omega], lr) + the step loop     (153-162)  optimize_splines(model, decoders, t_vals, steps, ...)
   compute_energy / compute_geodesic_lengths              compute_energy / compute_geodesic_lengths
      (src/single_decoder/optimize_energy_batched.py:42-57)
@@ -21,6 +23,7 @@ from __future__ import annotations
 from typing import Optional, Sequence
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib, ops
 
@@ -105,9 +108,66 @@ class DecoderEnsemble:
         return self.packed.device
 
 
+def _refuse_untracked_grads(what: str, **tensors) -> None:
+    """Gradients flow to omega, a and b only: refuse instead of leaving .grad of anything else at None."""
+    if torch.is_grad_enabled():
+        for name, x in tensors.items():
+            if x.requires_grad:
+                raise _lib.VlgError(f"{what}: no gradient with respect to {name} (only omega, a and b are differentiable)")
+
+
+def _wants_grad(model) -> bool:
+    return torch.is_grad_enabled() and (model.omega.requires_grad or model.a.requires_grad or model.b.requires_grad)
+
+
+class _SplinePoints(torch.autograd.Function):
+    """z = GeodesicSplineBatch.forward(t); backward by vlg_spline_points_backward (z is linear in omega, a, b)."""
+
+    @staticmethod
+    def forward(ctx, omega, a, b, basis, t, n_poly):
+        z = torch.empty((t.shape[0], omega.shape[0], 2), dtype=torch.float32, device=omega.device)
+        ops.spline_points(n_poly, a, b, omega, basis, t, z)
+        ctx.save_for_backward(basis, t)
+        ctx.n_poly, ctx.N, ctx.Kb = n_poly, omega.shape[0], omega.shape[1]
+        return z
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dz):
+        basis, t = ctx.saved_tensors
+        go = torch.empty((ctx.N, ctx.Kb, 2), dtype=torch.float32, device=dz.device)
+        ga = torch.empty((ctx.N, 2), dtype=torch.float32, device=dz.device)
+        gb = torch.empty_like(ga)
+        ops.spline_points_backward(ctx.n_poly, basis, t, dz.contiguous().float(), go, ga, gb)
+        return go, ga, gb, None, None, None
+
+
+class _CurveEnergy(torch.autograd.Function):
+    """Energy [N] with the gradients one vlg_curve_energy_grad launch formed next to it; the backward only
+    scales them by the incoming dL/dE[n]."""
+
+    @staticmethod
+    def forward(ctx, omega, a, b, launch):
+        energy, g_omega, g_a, g_b = launch()
+        ctx.save_for_backward(g_omega, g_a, g_b)
+        return energy
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_e):
+        g_omega, g_a, g_b = ctx.saved_tensors
+        ge = grad_e.to(torch.float32)
+        need = ctx.needs_input_grad
+        return (ge[:, None, None] * g_omega if need[0] else None, ge[:, None] * g_a if need[1] else None,
+                ge[:, None] * g_b if need[2] else None, None)
+
+
 class GeodesicSplineBatch:
     """Endpoint-constrained piecewise-cubic curves z_b(t) (src/optimize.py:13-35).
-    Holds omega [N,Kb,2] (updated in place by optimize_splines) and the Adam state."""
+    Holds omega [N,Kb,2] (updated in place by optimize_splines) and the Adam state.
+
+    omega, a and b are plain tensors; mark them ``requires_grad_()`` to differentiate forward(t) and
+    compute_energy_mc with torch.autograd (the reference's nn.Parameter omega, src/optimize.py:20)."""
 
     def __init__(self, a, b, basis, omega, n_poly: int):
         self.a = a.contiguous().float()
@@ -120,8 +180,12 @@ class GeodesicSplineBatch:
         self.step_count = 0
 
     def forward(self, t: torch.Tensor) -> torch.Tensor:
+        t = t.contiguous().float()
+        _refuse_untracked_grads("GeodesicSplineBatch.forward", basis=self.basis, t=t)
+        if _wants_grad(self):
+            return _SplinePoints.apply(self.omega, self.a, self.b, self.basis, t, self.n_poly)
         z = torch.empty((t.shape[0], self.omega.shape[0], 2), dtype=torch.float32, device=self.omega.device)
-        ops.spline_points(self.n_poly, self.a, self.b, self.omega, self.basis, t.contiguous().float(), z)
+        ops.spline_points(self.n_poly, self.a, self.b, self.omega, self.basis, t, z)
         return z
 
     __call__ = forward
@@ -247,11 +311,37 @@ def optimize_splines(model: GeodesicSplineBatch, decoders: DecoderEnsemble, t_va
 def compute_energy_mc(model: GeodesicSplineBatch, decoders: DecoderEnsemble, t_vals: torch.Tensor, M: int = 2,
                       draws=None, seed: int = 0, step: int = 0, curve_id0: int = 0, precision: str = "fp32",
                       return_length: bool = False, check: bool = True):
-    """MC ensemble curve energy [N] (src/optimize.py:38-75), forward only."""
+    """MC ensemble curve energy [N] (src/optimize.py:38-75).
+
+    Differentiable in model.omega, model.a and model.b: when grad mode is on and any of them requires grad, ONE
+    launch of the step kernel in gradient-output mode forms the energy and dE/d(omega), dE/da, dE/db (no penalty
+    term), and the result carries a grad_fn whose backward only scales them (once differentiable).  Otherwise a
+    forward-only launch.  The poly-line length (return_length) has no gradient."""
     N = model.omega.shape[0]
     T = t_vals.shape[0]
     prec = _resolve_precision(precision, decoders, M)
     dev = model.omega.device
+    _refuse_untracked_grads("compute_energy_mc", basis=model.basis, t_vals=t_vals)
+    if _wants_grad(model):
+        if return_length:
+            raise _lib.VlgError("compute_energy_mc: return_length=True has no gradient; evaluate lengths under "
+                                "torch.no_grad() (as src/single_decoder/optimize_energy_batched.py:42-49 does)")
+
+        def launch():
+            energy = torch.empty(N, dtype=torch.float32, device=dev)
+            g_omega = torch.empty_like(model.omega, dtype=torch.float32)
+            g_a = torch.empty((N, 2), dtype=torch.float32, device=dev)
+            g_b = torch.empty((N, 2), dtype=torch.float32, device=dev)
+            ws = _workspace(model, decoders, T, M, prec)
+            ops.curve_energy_grad(decoders.packed, decoders.K, decoders.X, len(decoders), model.n_poly, M,
+                                  model.a.detach(), model.b.detach(), model.omega.detach(), model.basis,
+                                  t_vals.contiguous().float(), _prep_draws(draws, N, 1, M, T, dev, len(decoders)),
+                                  None, seed, curve_id0, step, energy, g_omega, g_a, g_b, prec, ws)
+            if check:
+                _raise_on_status(ws, "compute_energy_mc")
+            return energy, g_omega, g_a, g_b
+
+        return _CurveEnergy.apply(model.omega, model.a, model.b, launch)
     energy = torch.empty(N, dtype=torch.float32, device=dev)
     length = torch.empty(N, dtype=torch.float32, device=dev) if return_length else None
     ws = _workspace(model, decoders, T, M, prec)

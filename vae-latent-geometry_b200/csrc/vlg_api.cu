@@ -199,6 +199,41 @@ int vlg_curve_energy(const void* packed, int K, int X, int K_active, int N, int 
   return dispatch(p, false, st);
 }
 
+int vlg_curve_energy_grad(const void* packed, int K, int X, int K_active, int N, int T, int n_poly, int M,
+                          const float* a, const float* b, const float* omega, const float* basis, const float* t,
+                          const uint8_t* draws, const int32_t* decoder_base, uint64_t seed, int64_t curve_id0, int step,
+                          float* energy, float* grad_omega, float* grad_a, float* grad_b, int precision,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+  if (!a || !b || !omega || !basis || !t || !energy || !grad_omega || !grad_a || !grad_b || step < 0)
+    return VLG_ERR_INVALID_ARGUMENT;
+  int rc = check_device();
+  if (rc != VLG_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  vlg::StepParams p;
+  rc = fill_params(&p, packed, K, X, K_active, N, T, n_poly, M, precision);
+  if (rc != VLG_OK) return rc;
+  if (workspace_bytes < vlg_workspace_bytes(N, T, n_poly, K_active, M, precision)) return VLG_ERR_WORKSPACE;
+  // one step of the optimiser's kernel in gradient-output mode: same draw stream as vlg_curve_energy at `step`
+  p.steps = 1;
+  p.step0 = step;
+  p.a = a;
+  p.b = b;
+  p.omega = const_cast<float*>(omega);   // read only in gradient-output mode
+  p.basis = basis;
+  p.t = t;
+  p.draws = draws;
+  p.dec_base = decoder_base;
+  p.seed = seed;
+  p.curve_id0 = curve_id0;
+  p.energy_last = energy;
+  p.grad_omega = grad_omega;
+  p.grad_a = grad_a;
+  p.grad_b = grad_b;
+  p.workspace = workspace;
+  p.workspace_bytes = workspace_bytes;
+  return dispatch(p, true, st);
+}
+
 int vlg_ensemble_std_norm(const void* packed, int K, int X, int K_active, int G, const float* grid, float* out,
                           void* stream) {
   if (!packed || !grid || !out || G <= 0 || K_active < 1) return VLG_ERR_INVALID_ARGUMENT;
@@ -217,6 +252,18 @@ int vlg_spline_points(int N, int T, int n_poly, const float* a, const float* b, 
   int rc = check_device();
   if (rc != VLG_OK) return rc;
   cudaError_t e = vlg::launch_spline_points(N, T, n_poly, a, b, omega, basis, t, z, static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? VLG_OK : cuda_fail(e);
+}
+
+int vlg_spline_points_backward(int N, int T, int n_poly, const float* basis, const float* t, const float* dz,
+                               float* grad_omega, float* grad_a, float* grad_b, void* stream) {
+  if (!basis || !t || !dz || !grad_omega || !grad_a || !grad_b || N <= 0 || T <= 0 || n_poly < 1)
+    return VLG_ERR_INVALID_ARGUMENT;
+  if (n_poly > vlg::MAX_NPOLY) return VLG_ERR_UNSUPPORTED;
+  int rc = check_device();
+  if (rc != VLG_OK) return rc;
+  cudaError_t e = vlg::launch_spline_points_backward(N, T, n_poly, basis, t, dz, grad_omega, grad_a, grad_b,
+                                                     static_cast<cudaStream_t>(stream));
   return e == cudaSuccess ? VLG_OK : cuda_fail(e);
 }
 

@@ -31,6 +31,11 @@ struct StepParams {
   float* energy_last;          // [N] or null
   float* energy_trace;         // [steps][N] or null
   float* length_out;           // [N] or null (forward-only mode)
+  // gradient-output mode (vlg_curve_energy_grad; null otherwise): the GRAD kernels write dE/d(omega), dE/da and
+  // dE/db of the energy alone (no penalty term) and skip Adam; omega is read only, adam_m / adam_v are null
+  float* grad_omega;           // [N,Kb,2]
+  float* grad_a;               // [N,2]
+  float* grad_b;               // [N,2]
   void* workspace;
   size_t workspace_bytes;
   int precision;
@@ -49,6 +54,8 @@ cudaError_t launch_std_norm(const void* packed, int K, int X, int G, const float
                             cudaStream_t stream);
 cudaError_t launch_spline_points(int N, int T, int n_poly, const float* a, const float* b, const float* omega,
                                  const float* basis, const float* t, float* z, cudaStream_t stream);
+cudaError_t launch_spline_points_backward(int N, int T, int n_poly, const float* basis, const float* t, const float* dz,
+                                          float* grad_omega, float* grad_a, float* grad_b, cudaStream_t stream);
 cudaError_t launch_fit_splines(int N, int Lmax, int n_poly, const float* targets, const int32_t* lens,
                                const float* basis, float* omega, float* ab, cudaStream_t stream);
 

@@ -1,5 +1,5 @@
-// Weight repacking and the small forward-only helpers (disagreement field, spline
-// evaluation, least-squares spline fit).  None of these are hot; they exist so the
+// Weight repacking and the small helpers (disagreement field, spline evaluation and its
+// backward, least-squares spline fit).  None of these are hot; they exist so the
 // drop-in entry points never leave the GPU and never need a CPU fallback.
 #include <cuda_fp16.h>
 
@@ -170,6 +170,54 @@ __global__ void spline_points_kernel(int N, int T, int n_poly, const float* __re
   }
 }
 
+// Backward of spline_points_kernel: z[t] = (1-t) a + t b + P[t] omega is linear in (omega, a, b), so
+// d(omega) = sum_t P[t]^T dz[t], da = sum_t (1-t) dz[t], db = sum_t t dz[t].  One block per curve; each thread sums
+// its points in order, then the warps and the block reduce in a fixed order: repeated calls give the same bits.
+__global__ void __launch_bounds__(256) spline_points_backward_kernel(int N, int T, int n_poly,
+                                                                     const float* __restrict__ basis,
+                                                                     const float* __restrict__ t,
+                                                                     const float* __restrict__ dz,
+                                                                     float* __restrict__ grad_omega,
+                                                                     float* __restrict__ grad_a,
+                                                                     float* __restrict__ grad_b) {
+  constexpr int NCOL = 2 * MAX_KB + 4;   // 2 Kb columns of P^T dz, then (1-t) dz and t dz
+  __shared__ float red[8][NCOL];
+  const int n = blockIdx.x, Kb = n_poly + 1, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  float acc[NCOL];
+#pragma unroll
+  for (int c = 0; c < NCOL; ++c) acc[c] = 0.f;
+  for (int i = threadIdx.x; i < T; i += blockDim.x) {
+    const float ti = t[i];
+    const float dx = dz[(size_t(i) * N + n) * 2], dy = dz[(size_t(i) * N + n) * 2 + 1];
+    float P[MAX_KB];
+    design_row(ti, n_poly, Kb, basis, P);
+#pragma unroll
+    for (int k = 0; k < MAX_KB; ++k)
+      if (k < Kb) {
+        acc[2 * k] = fmaf(P[k], dx, acc[2 * k]);
+        acc[2 * k + 1] = fmaf(P[k], dy, acc[2 * k + 1]);
+      }
+    acc[NCOL - 4] = fmaf(1.0f - ti, dx, acc[NCOL - 4]);
+    acc[NCOL - 3] = fmaf(1.0f - ti, dy, acc[NCOL - 3]);
+    acc[NCOL - 2] = fmaf(ti, dx, acc[NCOL - 2]);
+    acc[NCOL - 1] = fmaf(ti, dy, acc[NCOL - 1]);
+  }
+#pragma unroll
+  for (int c = 0; c < NCOL; ++c) {
+    const float v = warp_sum(acc[c]);
+    if (lane == 0) red[warp][c] = v;
+  }
+  __syncthreads();
+  const int c = threadIdx.x;
+  if (c < NCOL && (c < 2 * Kb || c >= NCOL - 4)) {
+    float g = 0.f;
+    for (int w = 0; w < 8; ++w) g += red[w][c];
+    if (c < 2 * Kb) grad_omega[size_t(n) * 2 * Kb + c] = g;
+    else if (c < NCOL - 2) grad_a[2 * n + c - (NCOL - 4)] = g;
+    else grad_b[2 * n + c - (NCOL - 2)] = g;
+  }
+}
+
 // ---- least-squares fit of the spline to a poly-line (init_splines_ensemble.py:172-193) ----
 // one warp per curve; normal equations in double, Gaussian elimination with pivoting.
 __global__ void __launch_bounds__(32) fit_splines_kernel(int N, int Lmax, int n_poly,
@@ -252,6 +300,12 @@ cudaError_t launch_std_norm(const void* packed, int K, int X, int G, const float
 cudaError_t launch_spline_points(int N, int T, int n_poly, const float* a, const float* b, const float* omega,
                                  const float* basis, const float* t, float* z, cudaStream_t stream) {
   spline_points_kernel<<<N, 256, 0, stream>>>(N, T, n_poly, a, b, omega, basis, t, z);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_spline_points_backward(int N, int T, int n_poly, const float* basis, const float* t, const float* dz,
+                                          float* grad_omega, float* grad_a, float* grad_b, cudaStream_t stream) {
+  spline_points_backward_kernel<<<N, 256, 0, stream>>>(N, T, n_poly, basis, t, dz, grad_omega, grad_a, grad_b);
   return cudaGetLastError();
 }
 

@@ -203,8 +203,11 @@ size_t simt_workspace_bytes(int N, int T, int K, int M) {
   return 256 + size_t(simt_grid(N)) * simt_max_items(W, K, M) * 2048;   // 256-byte header: word [1] = status flags
 }
 
-template <bool GRAD>
+// GOUT: gradient-output mode (vlg_curve_energy_grad, GRAD only): energy and dE/d(omega), dE/da, dE/db out, no Adam.
+// A template parameter, not a runtime branch, so that the optimiser's instantiation carries none of its code.
+template <bool GRAD, bool GOUT>
 __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, int W, int max_items) {
+  static_assert(GRAD || !GOUT, "gradient-output mode runs the backward items");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4, lane = tid & 31, warp = tid >> 5;
   const int M = p.M, K = p.K, T = p.T, n_poly = p.n_poly, Kb = p.Kb, X = p.X;
@@ -215,13 +218,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
   if (blockIdx.x == 0 && tid == 0 && !packed_header_ok(p.packed, p.K_total, p.X)) atomicOr(status, unsigned(VLG_STATUS_BAD_PACKED));
   const int WSEG = W - 1;
   const int nwin = (T - 1 + WSEG - 1) / WSEG;
+  // gradient-output mode: dE/da, dE/db accumulate in the Adam-moment slots of s.om, which this mode does not use
+  constexpr bool gout = GOUT;
+  float* gab = s.om + 2 * MAX_KB;
   for (int i = tid; i < 4 * n_poly * Kb; i += NTHREADS) s.basis[i] = p.basis[i];
 
   for (int n = blockIdx.x; n < p.N; n += gridDim.x) {
   // ---- per-curve state -> shared ----
   if (tid < 2 * Kb) {
     s.om[tid] = p.omega[size_t(n) * 2 * Kb + tid];
-    if (GRAD) {
+    if (GRAD && !gout) {
       s.om[2 * MAX_KB + tid] = p.adam_m[size_t(n) * 2 * Kb + tid];
       s.om[4 * MAX_KB + tid] = p.adam_v[size_t(n) * 2 * Kb + tid];
     }
@@ -245,6 +251,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
       s.coef[tid] = acc;
     }
     if (tid < 2 * MAX_KB) s.gacc[tid] = 0.f;
+    if (gout && tid < 4) gab[tid] = 0.f;
     float e_tot = 0.f, l_tot = 0.f;  // meaningful in thread 0
     __syncthreads();
 
@@ -507,8 +514,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
           const int pt = base + tid;
           float P[MAX_KB];
           float2 dz = make_float2(0.f, 0.f);
+          float tp = 0.f;
           if (pt < W) {
-            design_row(s.ts[pt], n_poly, Kb, s.basis, P);
+            tp = s.ts[pt];
+            design_row(tp, n_poly, Kb, s.basis, P);
             dz = s.dzs[pt];
           } else {
 #pragma unroll
@@ -527,6 +536,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
             s.gacc[tid] += g;
           }
           __syncthreads();
+          if (gout) {   // dE/da += sum (1-t) dz, dE/db += sum t dz: the design row extended by (1-t, t), second pass
+            const float ax = warp_sum((1.0f - tp) * dz.x), ay = warp_sum((1.0f - tp) * dz.y);
+            const float bx = warp_sum(tp * dz.x), by = warp_sum(tp * dz.y);
+            if (lane == 0) { s.red[warp * 20] = ax; s.red[warp * 20 + 1] = ay; s.red[warp * 20 + 2] = bx; s.red[warp * 20 + 3] = by; }
+            __syncthreads();
+            if (tid < 4) {
+              float g = 0.f;
+              for (int w = 0; w < 8; ++w) g += s.red[w * 20 + tid];
+              gab[tid] += g;
+            }
+            __syncthreads();
+          }
         }
       }
     }  // windows
@@ -541,7 +562,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
         if (p.length_out) p.length_out[n] = l_tot / float(M);
       }
     }
-    if (GRAD && tid < 2 * Kb) {
+    if (gout && tid < 2 * Kb + 4) {
+      // dE/d(omega), dE/da, dE/db of the energy alone
+      const float g = tid < 2 * Kb ? s.gacc[tid] : gab[tid - 2 * Kb];
+      if (!(fabsf(g) <= 3.0e38f)) atomicOr(status, unsigned(VLG_STATUS_NONFINITE));
+      if (tid < 2 * Kb) p.grad_omega[size_t(n) * 2 * Kb + tid] = g;
+      else if (tid < 2 * Kb + 2) p.grad_a[2 * n + tid - 2 * Kb] = g;
+      else p.grad_b[2 * n + tid - 2 * Kb - 2] = g;
+    } else if (GRAD && !gout && tid < 2 * Kb) {
       const int k = tid >> 1, d = tid & 1;
       const float tend = p.t[T - 1];
       float P[MAX_KB];
@@ -559,7 +587,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
     __syncthreads();
   }  // steps
 
-  if (GRAD && tid < 2 * Kb) {
+  if (GRAD && !gout && tid < 2 * Kb) {
     p.omega[size_t(n) * 2 * Kb + tid] = s.om[tid];
     p.adam_m[size_t(n) * 2 * Kb + tid] = s.om[2 * MAX_KB + tid];
     p.adam_v[size_t(n) * 2 * Kb + tid] = s.om[4 * MAX_KB + tid];
@@ -578,16 +606,14 @@ cudaError_t launch_simt(const StepParams& p, bool grad, cudaStream_t stream) {
   if (p.workspace == nullptr || p.workspace_bytes < simt_workspace_bytes(p.N, p.T, p.K, p.M)) return cudaErrorInvalidValue;
   cudaError_t e = cudaMemsetAsync(p.workspace, 0, 256, stream);
   if (e != cudaSuccess) return e;
-  if (grad) {
-    e = cudaFuncSetAttribute(simt_curve_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-    if (e != cudaSuccess) return e;
-    simt_curve_kernel<true><<<grid, NTHREADS, smem, stream>>>(p, W, max_items);
-  } else {
-    e = cudaFuncSetAttribute(simt_curve_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-    if (e != cudaSuccess) return e;
-    simt_curve_kernel<false><<<grid, NTHREADS, smem, stream>>>(p, W, max_items);
-  }
-  return cudaGetLastError();
+  auto launch = [&](auto kernel) -> cudaError_t {
+    cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (err != cudaSuccess) return err;
+    kernel<<<grid, NTHREADS, smem, stream>>>(p, W, max_items);
+    return cudaGetLastError();
+  };
+  if (grad && p.grad_omega) return launch(simt_curve_kernel<true, true>);
+  return grad ? launch(simt_curve_kernel<true, false>) : launch(simt_curve_kernel<false, false>);
 }
 
 }  // namespace vlg

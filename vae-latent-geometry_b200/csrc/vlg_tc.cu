@@ -361,8 +361,11 @@ static int tc_stages(int W, int K, int M, int xl2) {
   return int(nst);
 }
 
-template <bool GRAD, int FMT, bool XL2>
+// GOUT: gradient-output mode (vlg_curve_energy_grad, GRAD only): energy and dE/d(omega), dE/da, dE/db out, no Adam.
+// A template parameter, not a runtime branch, so that the optimiser's instantiations carry none of its code.
+template <bool GRAD, int FMT, bool XL2, bool GOUT>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, int nst, int W, int G_) {
+  static_assert(GRAD || !GOUT, "gradient-output mode runs the backward items");
   constexpr bool xl2 = XL2;               // left-end outputs / differences in the L2 workspace instead of shared memory
   constexpr int GM = XL2 ? TC_MAX_G : 1;  // curves per window this kernel is built for
   const int G = XL2 ? G_ : 1;             // curves per window of this launch: G > 1 = G whole curves (W = G T points)
@@ -699,7 +702,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
         if (j < Gcur) {
           const size_t o = size_t(n0 + j) * 2 * Kb + c;
           s.om[j * OM_STRIDE + c] = __ldcg(p.omega + o);
-          if (GRAD) {
+          if (GRAD && !GOUT) {
             s.om[j * OM_STRIDE + 2 * MAX_KB + c] = __ldcg(p.adam_m + o);
             s.om[j * OM_STRIDE + 4 * MAX_KB + c] = __ldcg(p.adam_v + o);
           }
@@ -722,6 +725,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
           s.coef[j * 64 + q] = acc;
         }
         if (t512 < G * 20) s.gacc[t512] = 0.f;
+        // gradient-output mode: dE/da, dE/db of curve j accumulate in the Adam-moment slots of s.om, unused there
+        if (GOUT && t512 < G * 4) s.om[(t512 >> 2) * OM_STRIDE + 2 * MAX_KB + (t512 & 3)] = 0.f;
         if (t512 < G * 2) s.etot[t512] = 0.f;
         named_bar(3, EPI_THREADS);
         PH(16);
@@ -1386,6 +1391,32 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
               }
               named_bar(3, EPI_THREADS);
             }
+            // gradient-output mode: dE/da += sum (1-t) dz, dE/db += sum t dz -- the design row extended by (1-t, t),
+            // in a second pass of the same shape
+            if (GOUT) {
+              for (int ch = 0; ch < nchunk; ++ch) {
+                const int pt = ch * 512 + t512;
+                float dx = 0.f, dy = 0.f, tp = 0.f;
+                if (pt < W) {
+                  tp = p.t[min(seg0 + pt - (pt / Wp) * Wp, T - 1)];
+                  const float2 d0 = s.dzs[pt], d1 = s.dzs[W + pt], d2 = s.dzs[2 * W + pt], d3 = s.dzs[3 * W + pt];
+                  dx = (d0.x + d1.x) + (d2.x + d3.x);
+                  dy = (d0.y + d1.y) + (d2.y + d3.y);
+                }
+                const float ax = warp_sum((1.0f - tp) * dx), ay = warp_sum((1.0f - tp) * dy);
+                const float bx = warp_sum(tp * dx), by = warp_sum(tp * dy);
+                float* r = s.red + wpos * 20;
+                if (lane == 0) { r[0] = ax; r[1] = ay; r[2] = bx; r[3] = by; }
+                named_bar(3, EPI_THREADS);
+                if (t512 < 4) {
+                  for (int w = 0; w < 16; ++w) {
+                    const int p0 = ch * 512 + w * 32;
+                    if (p0 < W) s.om[(p0 / Wp) * OM_STRIDE + 2 * MAX_KB + t512] += s.red[w * 20 + t512];
+                  }
+                }
+                named_bar(3, EPI_THREADS);
+              }
+            }
           } else {
             named_bar(3, EPI_THREADS);
           }
@@ -1403,7 +1434,18 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
             if (p.length_out) p.length_out[n] = s.etot[2 * t512 + 1] / float(Mtot);
           }
         }
-        if (GRAD && t512 < Gcur * 2 * Kb) {
+        if (GOUT) {
+          // dE/d(omega), dE/da, dE/db of the energy alone
+          const int ncol = 2 * Kb + 4;
+          if (t512 < Gcur * ncol) {
+            const int j = t512 / ncol, c = t512 - j * ncol, n = n0 + j;
+            const float g = c < 2 * Kb ? s.gacc[j * 20 + c] : s.om[j * OM_STRIDE + 2 * MAX_KB + c - 2 * Kb];
+            if (!(fabsf(g) <= 3.0e38f)) atomicOr(&queue[1], unsigned(VLG_STATUS_NONFINITE));
+            if (c < 2 * Kb) p.grad_omega[size_t(n) * 2 * Kb + c] = g;
+            else if (c < 2 * Kb + 2) p.grad_a[2 * n + c - 2 * Kb] = g;
+            else p.grad_b[2 * n + c - 2 * Kb - 2] = g;
+          }
+        } else if (GRAD && t512 < Gcur * 2 * Kb) {
           const int j = t512 / (2 * Kb), c = t512 - j * 2 * Kb;
           const int k = c >> 1, d = c & 1;
           const float tend = p.t[T - 1];
@@ -1425,7 +1467,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
         named_bar(3, EPI_THREADS);
       }  // steps
 
-      if (GRAD && t512 < Gcur * 2 * Kb) {
+      if (GRAD && !GOUT && t512 < Gcur * 2 * Kb) {
         const int j = t512 / (2 * Kb), c = t512 - j * 2 * Kb;
         const size_t o = size_t(n0 + j) * 2 * Kb + c;
         p.omega[o] = s.om[j * OM_STRIDE + c];
@@ -1728,19 +1770,20 @@ cudaError_t launch_tc(const StepParams& p, bool grad, cudaStream_t stream) {
     kernel<<<grid, TC_THREADS, smem, stream>>>(q, nst, W, G);
     return cudaGetLastError();
   };
-  auto by_fmt = [&](auto grad_c, auto xl2_c) -> cudaError_t {
-    constexpr bool G = decltype(grad_c)::value, X = decltype(xl2_c)::value;
-    if (fmt == FMT_TF32) return launch(tc_curve_kernel<G, FMT_TF32, X>);
-    if (fmt == FMT_F16) return launch(tc_curve_kernel<G, FMT_F16, X>);
+  auto by_fmt = [&](auto grad_c, auto xl2_c, auto gout_c) -> cudaError_t {
+    constexpr bool G = decltype(grad_c)::value, X = decltype(xl2_c)::value, O = decltype(gout_c)::value;
+    if (fmt == FMT_TF32) return launch(tc_curve_kernel<G, FMT_TF32, X, O>);
+    if (fmt == FMT_F16) return launch(tc_curve_kernel<G, FMT_F16, X, O>);
     if constexpr (G) {   // forward only: the mixed format IS the 3-term format
-      if (fmt == FMT_F16X3F) return launch(tc_curve_kernel<G, FMT_F16X3F, X>);
+      if (fmt == FMT_F16X3F) return launch(tc_curve_kernel<G, FMT_F16X3F, X, O>);
     }
-    return launch(tc_curve_kernel<G, FMT_F16X3, X>);
+    return launch(tc_curve_kernel<G, FMT_F16X3, X, O>);
   };
   using T_ = std::true_type;
   using F_ = std::false_type;
-  if (grad) return xl2 ? by_fmt(T_{}, T_{}) : by_fmt(T_{}, F_{});
-  return xl2 ? by_fmt(F_{}, T_{}) : by_fmt(F_{}, F_{});
+  if (grad && p.grad_omega) return xl2 ? by_fmt(T_{}, T_{}, T_{}) : by_fmt(T_{}, F_{}, T_{});
+  if (grad) return xl2 ? by_fmt(T_{}, T_{}, F_{}) : by_fmt(T_{}, F_{}, F_{});
+  return xl2 ? by_fmt(F_{}, T_{}, F_{}) : by_fmt(F_{}, F_{}, F_{});
 }
 
 }  // namespace vlg

@@ -137,6 +137,31 @@ def curve_energy(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, 
         _lib.check(_lib.load().vlg_curve_energy(*args), "vlg_curve_energy")
 
 
+@torch.library.custom_op("vlg::curve_energy_grad",
+                         mutates_args=("energy", "grad_omega", "grad_a", "grad_b", "workspace"))
+def curve_energy_grad(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, n_poly: int, M: int,
+                      a: torch.Tensor, b: torch.Tensor, omega: torch.Tensor, basis: torch.Tensor, t: torch.Tensor,
+                      draws: Optional[torch.Tensor], decoder_base: Optional[torch.Tensor], seed: int, curve_id0: int,
+                      step: int, energy: torch.Tensor, grad_omega: torch.Tensor, grad_a: torch.Tensor,
+                      grad_b: torch.Tensor, precision: int, workspace: Optional[torch.Tensor]) -> None:
+    N, Kb = omega.shape[0], omega.shape[1]
+    T = t.shape[0]
+    if Kb != n_poly + 1:
+        raise _lib.VlgError(f"omega has Kb={Kb}, expected n_poly+1={n_poly + 1}")
+    args = [_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active, N, T, n_poly, M,
+            _chk(a, "a", shape=(N, 2)), _chk(b, "b", shape=(N, 2)), _chk(omega, "omega", shape=(N, Kb, 2)),
+            _chk(basis, "basis", shape=(4 * n_poly, Kb)), _chk(t, "t", shape=(T,)),
+            _chk(draws, "draws", dtype=torch.uint8, shape=(N, 1, M, 2, T - 1)) if draws is not None else 0,
+            _chk(decoder_base, "decoder_base", dtype=torch.int32, shape=(N,)) if decoder_base is not None else 0,
+            seed & 0xFFFFFFFFFFFFFFFF, curve_id0, step, _chk(energy, "energy", shape=(N,)),
+            _chk(grad_omega, "grad_omega", shape=(N, Kb, 2)), _chk(grad_a, "grad_a", shape=(N, 2)),
+            _chk(grad_b, "grad_b", shape=(N, 2)), precision,
+            _chk(workspace, "workspace", dtype=torch.uint8) if workspace is not None else 0,
+            workspace.numel() if workspace is not None else 0, _stream(omega)]
+    with torch.cuda.device(omega.device):
+        _lib.check(_lib.load().vlg_curve_energy_grad(*args), "vlg_curve_energy_grad")
+
+
 @torch.library.custom_op("vlg::ensemble_std_norm", mutates_args=("out",))
 def ensemble_std_norm(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, grid: torch.Tensor,
                       out: torch.Tensor) -> None:
@@ -161,6 +186,21 @@ def spline_points(n_poly: int, a: torch.Tensor, b: torch.Tensor, omega: torch.Te
                                                  _chk(basis, "basis", shape=(4 * n_poly, Kb)),
                                                  _chk(t, "t", shape=(T,)), _chk(z, "z", shape=(T, N, 2)),
                                                  _stream(omega)), "vlg_spline_points")
+
+
+@torch.library.custom_op("vlg::spline_points_backward", mutates_args=("grad_omega", "grad_a", "grad_b"))
+def spline_points_backward(n_poly: int, basis: torch.Tensor, t: torch.Tensor, dz: torch.Tensor,
+                           grad_omega: torch.Tensor, grad_a: torch.Tensor, grad_b: torch.Tensor) -> None:
+    N, Kb = grad_omega.shape[0], grad_omega.shape[1]
+    T = t.shape[0]
+    with torch.cuda.device(dz.device):
+        _lib.check(_lib.load().vlg_spline_points_backward(N, T, n_poly,
+                                                          _chk(basis, "basis", shape=(4 * n_poly, Kb)),
+                                                          _chk(t, "t", shape=(T,)), _chk(dz, "dz", shape=(T, N, 2)),
+                                                          _chk(grad_omega, "grad_omega", shape=(N, Kb, 2)),
+                                                          _chk(grad_a, "grad_a", shape=(N, 2)),
+                                                          _chk(grad_b, "grad_b", shape=(N, 2)), _stream(dz)),
+                   "vlg_spline_points_backward")
 
 
 @torch.library.custom_op("vlg::fit_splines", mutates_args=("omega", "ab"))
