@@ -21,7 +21,7 @@
  *
  * Shapes (names follow the reference): N curves, T points per curve (t grid), n_poly
  * cubic segments, Kb = n_poly+1 free coefficients per latent dim, K decoders
- * 2 -> H(=128) -> H -> X (X <= 64; 50 for tasic-pca50), M Monte-Carlo decoder pairings.
+ * 2 -> H(=128) -> H -> X (1 <= X <= 52; 50 for tasic-pca50), M Monte-Carlo decoder pairings.
  * Limits (VLG_ERR_UNSUPPORTED beyond them): n_poly <= 8; K_active <= 254 with VLG_PRECISION_FP32, <= 128 on the
  * tensor-core precisions; M <= 4 with VLG_PRECISION_FP32, <= 64 on the tensor-core precisions (blocks of two).
  */

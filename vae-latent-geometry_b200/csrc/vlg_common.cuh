@@ -6,7 +6,7 @@
 namespace vlg {
 
 constexpr int H = 128;          // hidden width of the decoder MLP (src/train.py:80-85)
-constexpr int XP = 64;          // padded output width (X <= 64; tasic-pca50: X = 50)
+constexpr int XP = 64;          // padded width of the W3 blocks; X itself is <= 52 (XD_STRIDE / DIFF_STRIDE); tasic-pca50: X = 50
 constexpr int TILE_ROWS = 128;  // curve points per tile (= MMA M, = TMEM lanes)
 constexpr int TILE_SEGS = 127;  // curve segments per tile: adjacent tiles share one point
 constexpr int MAX_NPOLY = 8;

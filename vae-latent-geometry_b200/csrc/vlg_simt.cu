@@ -24,7 +24,7 @@ namespace vlg {
 namespace {
 
 constexpr int NTHREADS = 256;
-constexpr int DIFF_STRIDE = 52;  // floats per (m,row) Diff vector (X<=50 padded; 16B rows)
+constexpr int DIFF_STRIDE = 52;  // floats per (m,row) Diff vector (X<=52; 16B rows)
 constexpr int BS_FLOATS = 16 * 128;
 
 // transposed + swizzled activation tile: element (k, row)
