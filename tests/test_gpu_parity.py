@@ -267,7 +267,8 @@ def test_errors_are_loud(vlg):
 @pytest.mark.parametrize("prec", ["fp32", "f16", "f16x3", "tf32"])
 def test_kernel_status_word_reports_bad_draws_and_overflow(vlg, prec):
     """The C ABI itself (no host-side validation): an out-of-range explicit draw is clamped and flagged, and
-    a non-finite result (fp16 operand overflow) is flagged -- vlg_workspace_status returns VLG_ERR_NUMERIC."""
+    a non-finite result (fp16 operand overflow, or an omega the Adam step made non-finite) is flagged --
+    vlg_workspace_status returns VLG_ERR_NUMERIC."""
     from vlg_b200 import ops, api
     g = Hh.load("synth_np4_T130")
     N, T, K, M = g["a"].shape[0], 130, 4, 2
@@ -275,18 +276,20 @@ def test_kernel_status_word_reports_bad_draws_and_overflow(vlg, prec):
     code = ops.PRECISIONS[prec]
     t = torch.linspace(0, 1, T, device="cuda")
 
-    def launch(dec_, draws):
+    def launch(dec_, draws, lr=1e-3):
         m = make_model(vlg, g)
         ws = api._workspace(m, dec_, T, M, code)
         e = torch.empty(N, device="cuda")
         ops.optimize_steps(dec_.packed, dec_.K, dec_.X, len(dec_), 4, M, 1, 0, m.a, m.b, m.omega, m.adam_m, m.adam_v,
-                           m.basis, t, draws, None, 0, 0, 1e-3, 0.9, 0.999, 1e-8, 1000.0, e, None, code, ws)
+                           m.basis, t, draws, None, 0, 0, lr, 0.9, 0.999, 1e-8, 1000.0, e, None, code, ws)
         return ops.workspace_status(ws), e
 
     assert launch(dec, None)[0] == 0
     bad = torch.full((N, 1, M, 2, T - 1), 200, dtype=torch.uint8, device="cuda")
     flags, e = launch(dec, bad)
     assert flags & ops.STATUS_BAD_DRAW and bool(torch.isfinite(e).all())     # clamped to decoder K-1, memory-safe
+    flags, e = launch(dec, None, lr=float("inf"))     # the energy before the step is finite, the stepped omega is not
+    assert flags & ops.STATUS_NONFINITE and bool(torch.isfinite(e).all())
     # decoders whose hidden activations exceed the fp16 range
     arrs = {k: v.copy() for k, v in Hh.decoder_arrays(g).items()}
     arrs["W2"] = arrs["W2"] * 3.0e4

@@ -322,33 +322,28 @@ def compute_energy_mc(model: GeodesicSplineBatch, decoders: DecoderEnsemble, t_v
     prec = _resolve_precision(precision, decoders, M)
     dev = model.omega.device
     _refuse_untracked_grads("compute_energy_mc", basis=model.basis, t_vals=t_vals)
-    if _wants_grad(model):
-        if return_length:
-            raise _lib.VlgError("compute_energy_mc: return_length=True has no gradient; evaluate lengths under "
-                                "torch.no_grad() (as src/single_decoder/optimize_energy_batched.py:42-49 does)")
-
+    grad = _wants_grad(model)
+    if grad and return_length:
+        raise _lib.VlgError("compute_energy_mc: return_length=True has no gradient; evaluate lengths under "
+                            "torch.no_grad() (as src/single_decoder/optimize_energy_batched.py:42-49 does)")
+    energy = torch.empty(N, dtype=torch.float32, device=dev)
+    ws = _workspace(model, decoders, T, M, prec)
+    args = (decoders.packed, decoders.K, decoders.X, len(decoders), model.n_poly, M, model.a.detach(),
+            model.b.detach(), model.omega.detach(), model.basis, t_vals.contiguous().float(),
+            _prep_draws(draws, N, 1, M, T, dev, len(decoders)), None, seed, curve_id0, step, energy)
+    if grad:
         def launch():
-            energy = torch.empty(N, dtype=torch.float32, device=dev)
-            g_omega = torch.empty_like(model.omega, dtype=torch.float32)
-            g_a = torch.empty((N, 2), dtype=torch.float32, device=dev)
-            g_b = torch.empty((N, 2), dtype=torch.float32, device=dev)
-            ws = _workspace(model, decoders, T, M, prec)
-            ops.curve_energy_grad(decoders.packed, decoders.K, decoders.X, len(decoders), model.n_poly, M,
-                                  model.a.detach(), model.b.detach(), model.omega.detach(), model.basis,
-                                  t_vals.contiguous().float(), _prep_draws(draws, N, 1, M, T, dev, len(decoders)),
-                                  None, seed, curve_id0, step, energy, g_omega, g_a, g_b, prec, ws)
+            grads = (torch.empty_like(model.omega, dtype=torch.float32),
+                     torch.empty((N, 2), dtype=torch.float32, device=dev),
+                     torch.empty((N, 2), dtype=torch.float32, device=dev))
+            ops.curve_energy_grad(*args, *grads, prec, ws)
             if check:
                 _raise_on_status(ws, "compute_energy_mc")
-            return energy, g_omega, g_a, g_b
+            return (energy, *grads)
 
         return _CurveEnergy.apply(model.omega, model.a, model.b, launch)
-    energy = torch.empty(N, dtype=torch.float32, device=dev)
     length = torch.empty(N, dtype=torch.float32, device=dev) if return_length else None
-    ws = _workspace(model, decoders, T, M, prec)
-    ops.curve_energy(decoders.packed, decoders.K, decoders.X, len(decoders), model.n_poly, M, model.a, model.b,
-                     model.omega, model.basis, t_vals.contiguous().float(),
-                     _prep_draws(draws, N, 1, M, T, dev, len(decoders)), None, seed, curve_id0, step,
-                     energy, length, prec, ws)
+    ops.curve_energy(*args, length, prec, ws)
     if check:
         _raise_on_status(ws, "compute_energy_mc")
     return (energy, length) if return_length else energy

@@ -1,11 +1,33 @@
 // extern "C" front end: argument validation, device check, dispatch.  See include/vlg.h.
 #include "../../include/vlg.h"
 
+#include <math.h>
 #include <stdio.h>
-#include <string.h>
 
 #include "vlg_common.cuh"
 #include "vlg_kernels.h"
+
+namespace vlg {
+
+int persistent_grid(int N) {
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) == cudaSuccess) {
+    int v = 0;
+    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && v > 0) sms = v;
+  } else {
+    (void)cudaGetLastError();
+  }
+  return N < sms ? N : sms;
+}
+
+double expected_items(int w, double p) {
+  const double mean = w * p, sd = sqrt(w * p * (1.0 - p)) + 1e-9;
+  double items = 0.0;
+  for (int q = 0; q * 128 < w; ++q) items += 0.5 * erfc((q * 128 + 0.5 - mean) / (sd * 1.4142135623730951));  // P(n > 128 q)
+  return items;
+}
+
+}  // namespace vlg
 
 namespace {
 
@@ -27,37 +49,45 @@ int check_device() {
   return VLG_OK;
 }
 
-int fill_params(vlg::StepParams* p, const void* packed, int K, int X, int K_active, int N, int T, int n_poly, int M,
-                int precision) {
+// What the three step entry points share: the device check, the shape and workspace checks, the fields every mode
+// sets, and the launch of the fp32 or the tensor-core kernel.  `p` comes with the mode, steps, step0 and the mode's
+// own fields set and all else zero; the caller has checked its own arguments.
+int launch_step(vlg::StepParams& p, const void* packed, int K, int X, int K_active, int N, int T, int n_poly, int M,
+                const float* a, const float* b, const float* omega, const float* basis, const float* t,
+                const uint8_t* draws, const int32_t* decoder_base, uint64_t seed, int64_t curve_id0, int precision,
+                void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = check_device();
+  if (rc != VLG_OK) return rc;
   if (!packed || N <= 0 || T < 2 || n_poly < 1 || M < 1 || K_active < 1) return VLG_ERR_INVALID_ARGUMENT;
   // MC samples: the fp32 kernel holds all of them at once (<= MAX_M); the tensor-core kernel walks blocks of two (<= 64)
   if (n_poly > vlg::MAX_NPOLY || M > (precision == VLG_PRECISION_FP32 ? vlg::MAX_M : 64) || K_active > 254) return VLG_ERR_UNSUPPORTED;
   if (precision < VLG_PRECISION_FP32 || precision > VLG_PRECISION_F16X3F) return VLG_ERR_INVALID_ARGUMENT;
   if (vlg_packed_decoders_bytes(K, vlg::H, X) == 0 || K_active > K) return VLG_ERR_INVALID_ARGUMENT;
-  memset(p, 0, sizeof(*p));
-  p->packed = packed;
-  p->K = K_active;
-  p->K_total = K;
-  p->X = X;
-  p->N = N;
-  p->T = T;
-  p->n_poly = n_poly;
-  p->Kb = n_poly + 1;
-  p->M = M;
-  p->precision = precision;
-  return VLG_OK;
-}
-
-int dispatch(const vlg::StepParams& p, bool grad, cudaStream_t stream) {
-  cudaError_t e;
-  if (p.precision == VLG_PRECISION_FP32) {
-    if (vlg::simt_smem_bytes(p.T, p.K, p.M) > 232448) return VLG_ERR_UNSUPPORTED;
-    e = vlg::launch_simt(p, grad, stream);
-    if (e == cudaErrorNotSupported) return VLG_ERR_UNSUPPORTED;
-  } else {
-    e = vlg::launch_tc(p, grad, stream);
-    if (e == cudaErrorNotSupported) return VLG_ERR_UNSUPPORTED;
-  }
+  if (workspace_bytes < vlg_workspace_bytes(N, T, n_poly, K_active, M, precision)) return VLG_ERR_WORKSPACE;
+  p.packed = packed;
+  p.K = K_active;
+  p.K_total = K;
+  p.X = X;
+  p.N = N;
+  p.T = T;
+  p.n_poly = n_poly;
+  p.Kb = n_poly + 1;
+  p.M = M;
+  p.a = a;
+  p.b = b;
+  p.omega = const_cast<float*>(omega);   // written only by StepMode::Optimize
+  p.basis = basis;
+  p.t = t;
+  p.draws = draws;
+  p.dec_base = decoder_base;
+  p.seed = seed;
+  p.curve_id0 = curve_id0;
+  p.workspace = workspace;
+  p.workspace_bytes = workspace_bytes;
+  p.precision = precision;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const cudaError_t e = precision == VLG_PRECISION_FP32 ? vlg::launch_simt(p, st) : vlg::launch_tc(p, st);
+  if (e == cudaErrorNotSupported) return VLG_ERR_UNSUPPORTED;
   return e == cudaSuccess ? VLG_OK : cuda_fail(e);
 }
 
@@ -112,26 +142,12 @@ int vlg_optimize_steps(const void* packed, int K, int X, int K_active, int N, in
   if (!a || !b || !omega || !adam_m || !adam_v || !basis || !t || steps < 0 || step0 < 0)
     return VLG_ERR_INVALID_ARGUMENT;
   if (steps == 0) return VLG_OK;
-  int rc = check_device();
-  if (rc != VLG_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  vlg::StepParams p;
-  rc = fill_params(&p, packed, K, X, K_active, N, T, n_poly, M, precision);
-  if (rc != VLG_OK) return rc;
-  if (workspace_bytes < vlg_workspace_bytes(N, T, n_poly, K_active, M, precision)) return VLG_ERR_WORKSPACE;
+  vlg::StepParams p{};
+  p.mode = vlg::StepMode::Optimize;
   p.steps = steps;
   p.step0 = step0;
-  p.a = a;
-  p.b = b;
-  p.omega = omega;
   p.adam_m = adam_m;
   p.adam_v = adam_v;
-  p.basis = basis;
-  p.t = t;
-  p.draws = draws;
-  p.dec_base = decoder_base;
-  p.seed = seed;
-  p.curve_id0 = curve_id0;
   p.lr = lr;
   p.beta1 = beta1;
   p.beta2 = beta2;
@@ -142,9 +158,8 @@ int vlg_optimize_steps(const void* packed, int K, int X, int K_active, int N, in
   p.penalty_w = float(penalty_w);
   p.energy_last = energy_last;
   p.energy_trace = energy_trace;
-  p.workspace = workspace;
-  p.workspace_bytes = workspace_bytes;
-  return dispatch(p, true, st);
+  return launch_step(p, packed, K, X, K_active, N, T, n_poly, M, a, b, omega, basis, t, draws, decoder_base, seed,
+                     curve_id0, precision, workspace, workspace_bytes, stream);
 }
 
 int vlg_workspace_status(const void* workspace, int* flags, void* stream) {
@@ -174,29 +189,14 @@ int vlg_curve_energy(const void* packed, int K, int X, int K_active, int N, int 
                      const int32_t* decoder_base, uint64_t seed, int64_t curve_id0, int step, float* energy, float* length, int precision,
                      void* workspace, size_t workspace_bytes, void* stream) {
   if (!a || !b || !omega || !basis || !t || !energy || step < 0) return VLG_ERR_INVALID_ARGUMENT;
-  int rc = check_device();
-  if (rc != VLG_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  vlg::StepParams p;
-  rc = fill_params(&p, packed, K, X, K_active, N, T, n_poly, M, precision);
-  if (rc != VLG_OK) return rc;
-  if (workspace_bytes < vlg_workspace_bytes(N, T, n_poly, K_active, M, precision)) return VLG_ERR_WORKSPACE;
+  vlg::StepParams p{};
+  p.mode = vlg::StepMode::Energy;
   p.steps = 1;
   p.step0 = step;
-  p.a = a;
-  p.b = b;
-  p.omega = const_cast<float*>(omega);
-  p.basis = basis;
-  p.t = t;
-  p.draws = draws;
-  p.dec_base = decoder_base;
-  p.seed = seed;
-  p.curve_id0 = curve_id0;
   p.energy_last = energy;
   p.length_out = length;
-  p.workspace = workspace;
-  p.workspace_bytes = workspace_bytes;
-  return dispatch(p, false, st);
+  return launch_step(p, packed, K, X, K_active, N, T, n_poly, M, a, b, omega, basis, t, draws, decoder_base, seed,
+                     curve_id0, precision, workspace, workspace_bytes, stream);
 }
 
 int vlg_curve_energy_grad(const void* packed, int K, int X, int K_active, int N, int T, int n_poly, int M,
@@ -206,32 +206,17 @@ int vlg_curve_energy_grad(const void* packed, int K, int X, int K_active, int N,
                           void* workspace, size_t workspace_bytes, void* stream) {
   if (!a || !b || !omega || !basis || !t || !energy || !grad_omega || !grad_a || !grad_b || step < 0)
     return VLG_ERR_INVALID_ARGUMENT;
-  int rc = check_device();
-  if (rc != VLG_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  vlg::StepParams p;
-  rc = fill_params(&p, packed, K, X, K_active, N, T, n_poly, M, precision);
-  if (rc != VLG_OK) return rc;
-  if (workspace_bytes < vlg_workspace_bytes(N, T, n_poly, K_active, M, precision)) return VLG_ERR_WORKSPACE;
   // one step of the optimiser's kernel in gradient-output mode: same draw stream as vlg_curve_energy at `step`
+  vlg::StepParams p{};
+  p.mode = vlg::StepMode::EnergyGrad;
   p.steps = 1;
   p.step0 = step;
-  p.a = a;
-  p.b = b;
-  p.omega = const_cast<float*>(omega);   // read only in gradient-output mode
-  p.basis = basis;
-  p.t = t;
-  p.draws = draws;
-  p.dec_base = decoder_base;
-  p.seed = seed;
-  p.curve_id0 = curve_id0;
   p.energy_last = energy;
   p.grad_omega = grad_omega;
   p.grad_a = grad_a;
   p.grad_b = grad_b;
-  p.workspace = workspace;
-  p.workspace_bytes = workspace_bytes;
-  return dispatch(p, true, st);
+  return launch_step(p, packed, K, X, K_active, N, T, n_poly, M, a, b, omega, basis, t, draws, decoder_base, seed,
+                     curve_id0, precision, workspace, workspace_bytes, stream);
 }
 
 int vlg_ensemble_std_norm(const void* packed, int K, int X, int K_active, int G, const float* grid, float* out,

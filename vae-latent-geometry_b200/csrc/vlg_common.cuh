@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "vlg_kernels.h"
+
 namespace vlg {
 
 constexpr int H = 128;          // hidden width of the decoder MLP (src/train.py:80-85)
@@ -175,6 +177,89 @@ __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
+}
+
+// ---------------------------------------------------------------------------------------
+// Per-curve step code of both step kernels (vlg_simt.cu, vlg_tc.cu).  `status` is the launch's status word
+// (VLG_STATUS_* flags, word [1] of the workspace header).  A curve's optimiser state `om` holds omega, m and v
+// at offsets 0, 2 MAX_KB and 4 MAX_KB.
+// ---------------------------------------------------------------------------------------
+// fp16 operands overflow above 65504: inf/NaN reach the energy (forward), the gradient or omega (backward)
+__device__ __forceinline__ void flag_nonfinite(float x, unsigned int* status) {
+  if (!(fabsf(x) <= 3.0e38f)) atomicOr(status, unsigned(VLG_STATUS_NONFINITE));
+}
+
+// First decoder of curve n's weight set inside `packed`.  Out of range: 0 (memory safety), reported by the
+// thread that passes `report`.
+__device__ __forceinline__ int curve_dec_base(const StepParams& p, int n, bool report, unsigned int* status) {
+  int base = p.dec_base ? p.dec_base[n] : 0;
+  if (base < 0 || base + p.K > p.K_total) {
+    base = 0;
+    if (report) atomicOr(status, unsigned(VLG_STATUS_BAD_PACKED));
+  }
+  return base;
+}
+
+// Explicit draw [n][step][m][role][seg] of draws [N][steps][M][2][T-1].  A value >= K is clamped to K - 1 (memory
+// safety) and sets `bad`, which the kernel reports through the status word.  The sizes come as arguments rather than
+// through StepParams: the callers store draws as bytes, which may alias a StepParams reference and would force a
+// reload of every field per draw, where the kernels keep the sizes in registers.
+__device__ __forceinline__ uint8_t explicit_draw(const uint8_t* draws, int steps, int M, int T, int K, int n, int step,
+                                                 int m, int role, int seg, bool& bad) {
+  uint8_t v = draws[(((size_t(n) * steps + step) * M + m) * 2 + role) * size_t(T - 1) + seg];
+  if (v >= K) { v = uint8_t(K - 1); bad = true; }
+  return v;
+}
+
+// Energy of curve n at `step` from its sums over the M samples: the trace entry and, at the launch's last step,
+// the energy and poly-line length outputs.
+__device__ __forceinline__ void write_energy(const StepParams& p, int n, int step, float e_sum, float l_sum,
+                                             unsigned int* status) {
+  const float E = e_sum / float(p.M);
+  flag_nonfinite(E, status);
+  if (p.energy_trace) p.energy_trace[size_t(step) * p.N + n] = E;
+  if (step == p.steps - 1) {
+    if (p.energy_last) p.energy_last[n] = E;
+    if (p.length_out) p.length_out[n] = l_sum / float(p.M);
+  }
+}
+
+// Component c of curve n's gradient output (EnergyGrad): dE/d(omega) for c < 2 Kb, then dE/da, dE/db.
+__device__ __forceinline__ void write_grad(const StepParams& p, int n, int c, float g, unsigned int* status) {
+  const int Kb = p.Kb;
+  flag_nonfinite(g, status);
+  if (c < 2 * Kb) p.grad_omega[size_t(n) * 2 * Kb + c] = g;
+  else if (c < 2 * Kb + 2) p.grad_a[2 * n + c - 2 * Kb] = g;
+  else p.grad_b[2 * n + c - 2 * Kb - 2] = g;
+}
+
+// One optimiser step of coefficient c = 2 k + d of a curve (end points a, b; coef = basis @ omega): the energy
+// gradient g_energy plus that of the end-point penalty w |z(t_end) - b|^2, then Adam on om.
+__device__ __forceinline__ void penalty_adam_step(const StepParams& p, int step, int c, float g_energy,
+                                                  const float* basis, const float* coef, float2 pa, float2 pb,
+                                                  float* om) {
+  const int k = c >> 1, d = c & 1;
+  const float tend = p.t[p.T - 1];
+  float P[MAX_KB];
+  design_row(tend, p.n_poly, p.Kb, basis, P);
+  const float2 ze = spline_point(tend, p.n_poly, coef, pa, pb);
+  const float err = d == 0 ? ze.x - pb.x : ze.y - pb.y;
+  const float g = g_energy + (2.0f * p.penalty_w) * err * P[k];
+  AdamScalars sc = adam_scalars(p.step0 + step + 1, p.lr, p.beta1, p.beta2);
+  float w = om[c], mm = om[2 * MAX_KB + c], vv = om[4 * MAX_KB + c];
+  adam_update(w, mm, vv, g, sc, p.one_minus_b1, p.beta2f, p.one_minus_b2, p.eps);
+  om[c] = w;
+  om[2 * MAX_KB + c] = mm;
+  om[4 * MAX_KB + c] = vv;
+}
+
+// omega, m and v of coefficient c of curve n back to memory (Optimize)
+__device__ __forceinline__ void write_back(const StepParams& p, int n, int c, const float* om, unsigned int* status) {
+  const size_t o = size_t(n) * 2 * p.Kb + c;
+  p.omega[o] = om[c];
+  p.adam_m[o] = om[2 * MAX_KB + c];
+  p.adam_v[o] = om[4 * MAX_KB + c];
+  flag_nonfinite(om[c], status);
 }
 
 }  // namespace vlg

@@ -172,42 +172,24 @@ static int simt_window_points(int T, int K, int M) {
   for (int nwin = 1; nwin <= segs; ++nwin) {
     const int w = (segs + nwin - 1) / nwin + 1;
     if (w <= SIMT_MAX_W && simt_smem_bytes_w(w, K, M) <= 232448 && simt_max_items(w, K, M) <= SIMT_MAX_ITEMS) {
-      const double mean = w * p, sd = sqrt(w * p * (1.0 - p)) + 1e-9;
-      double items = 0.0;
-      for (int q = 0; q * 128 < w; ++q) items += 0.5 * erfc((q * 128 + 0.5 - mean) / (sd * 1.4142135623730951));
-      const double cost = nwin * (K * items + 0.25);
+      const double cost = nwin * (K * expected_items(w, p) + 0.25);
       if (cost < best) { best = cost; best_w = w; }
     }
     if (w <= 128) break;
   }
   return best_w;  // 0: does not fit
 }
-static int simt_grid(int N) {
-  int dev = 0, sms = 148;
-  if (cudaGetDevice(&dev) == cudaSuccess) {
-    int v = 0;
-    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && v > 0) sms = v;
-  } else {
-    (void)cudaGetLastError();
-  }
-  return N < sms ? N : sms;
-}
-size_t simt_smem_bytes(int T, int K, int M) {
-  const int W = simt_window_points(T, K, M);
-  return W ? simt_smem_bytes_w(W, K, M) : size_t(1) << 30;
-}
 // layer-2 ReLU mask bits [cta][item][128 rows][16 bytes], L2 resident
 size_t simt_workspace_bytes(int N, int T, int K, int M) {
   const int W = simt_window_points(T, K, M);
   if (W == 0) return 0;
-  return 256 + size_t(simt_grid(N)) * simt_max_items(W, K, M) * 2048;   // 256-byte header: word [1] = status flags
+  return 256 + size_t(persistent_grid(N)) * simt_max_items(W, K, M) * 2048;   // 256-byte header: word [1] = status flags
 }
 
-// GOUT: gradient-output mode (vlg_curve_energy_grad, GRAD only): energy and dE/d(omega), dE/da, dE/db out, no Adam.
-// A template parameter, not a runtime branch, so that the optimiser's instantiation carries none of its code.
-template <bool GRAD, bool GOUT>
+template <StepMode MODE>
 __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, int W, int max_items) {
-  static_assert(GRAD || !GOUT, "gradient-output mode runs the backward items");
+  constexpr bool GRAD = MODE != StepMode::Energy;       // backward items
+  constexpr bool GOUT = MODE == StepMode::EnergyGrad;   // gradient out instead of Adam
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4, lane = tid & 31, warp = tid >> 5;
   const int M = p.M, K = p.K, T = p.T, n_poly = p.n_poly, Kb = p.Kb, X = p.X;
@@ -219,7 +201,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
   const int WSEG = W - 1;
   const int nwin = (T - 1 + WSEG - 1) / WSEG;
   // gradient-output mode: dE/da, dE/db accumulate in the Adam-moment slots of s.om, which this mode does not use
-  constexpr bool gout = GOUT;
   float* gab = s.om + 2 * MAX_KB;
   for (int i = tid; i < 4 * n_poly * Kb; i += NTHREADS) s.basis[i] = p.basis[i];
 
@@ -227,18 +208,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
   // ---- per-curve state -> shared ----
   if (tid < 2 * Kb) {
     s.om[tid] = p.omega[size_t(n) * 2 * Kb + tid];
-    if (GRAD && !gout) {
+    if (MODE == StepMode::Optimize) {
       s.om[2 * MAX_KB + tid] = p.adam_m[size_t(n) * 2 * Kb + tid];
       s.om[4 * MAX_KB + tid] = p.adam_v[size_t(n) * 2 * Kb + tid];
     }
   }
   const float2 pa = make_float2(p.a[2 * n], p.a[2 * n + 1]);
   const float2 pb = make_float2(p.b[2 * n], p.b[2 * n + 1]);
-  int dec_base = p.dec_base ? p.dec_base[n] : 0;   // first decoder of this curve's weight set inside `packed`
-  if (dec_base < 0 || dec_base + K > p.K_total) {
-    dec_base = 0;
-    if (tid == 0) atomicOr(status, unsigned(VLG_STATUS_BAD_PACKED));
-  }
+  const int dec_base = curve_dec_base(p, n, tid == 0, status);
   const float coefm = 2.0f / float(M);
   __syncthreads();
 
@@ -251,7 +228,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
       s.coef[tid] = acc;
     }
     if (tid < 2 * MAX_KB) s.gacc[tid] = 0.f;
-    if (gout && tid < 4) gab[tid] = 0.f;
+    if (GOUT && tid < 4) gab[tid] = 0.f;
     float e_tot = 0.f, l_tot = 0.f;  // meaningful in thread 0
     __syncthreads();
 
@@ -268,12 +245,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
         if (p.draws != nullptr) {
           for (int m = 0; m < M; ++m)
             for (int role = 0; role < 2; ++role) {
-              uint8_t v = 255;
-              if (pt < nseg) {
-                v = p.draws[(((size_t(n) * p.steps + step) * M + m) * 2 + role) * size_t(T - 1) + seg0 + pt];
-                if (v >= K) { v = uint8_t(K - 1); bad_draw = true; }   // memory safety; reported through the status word
-              }
-              s.sel[(m * 2 + role) * W + pt] = v;
+              s.sel[(m * 2 + role) * W + pt] = pt < nseg ? explicit_draw(p.draws, p.steps, M, T, K, n, step, m, role, seg0 + pt, bad_draw) : 255;
             }
         } else {
           for (int jp = 0; jp < (M + 1) / 2; ++jp) {
@@ -536,7 +508,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
             s.gacc[tid] += g;
           }
           __syncthreads();
-          if (gout) {   // dE/da += sum (1-t) dz, dE/db += sum t dz: the design row extended by (1-t, t), second pass
+          if (GOUT) {   // dE/da += sum (1-t) dz, dE/db += sum t dz: the design row extended by (1-t, t), second pass
             const float ax = warp_sum((1.0f - tp) * dz.x), ay = warp_sum((1.0f - tp) * dz.y);
             const float bx = warp_sum(tp * dz.x), by = warp_sum(tp * dz.y);
             if (lane == 0) { s.red[warp * 20] = ax; s.red[warp * 20 + 1] = ay; s.red[warp * 20 + 2] = bx; s.red[warp * 20 + 3] = by; }
@@ -552,56 +524,24 @@ __global__ void __launch_bounds__(NTHREADS, 1) simt_curve_kernel(StepParams p, i
       }
     }  // windows
 
-    // ---- step epilogue: energy out, penalty gradient, Adam ----
-    if (tid == 0) {
-      const float E = e_tot / float(M);
-      if (!(fabsf(E) <= 3.0e38f)) atomicOr(status, unsigned(VLG_STATUS_NONFINITE));
-      if (p.energy_trace) p.energy_trace[size_t(step) * p.N + n] = E;
-      if (step == p.steps - 1) {
-        if (p.energy_last) p.energy_last[n] = E;
-        if (p.length_out) p.length_out[n] = l_tot / float(M);
-      }
-    }
-    if (gout && tid < 2 * Kb + 4) {
-      // dE/d(omega), dE/da, dE/db of the energy alone
-      const float g = tid < 2 * Kb ? s.gacc[tid] : gab[tid - 2 * Kb];
-      if (!(fabsf(g) <= 3.0e38f)) atomicOr(status, unsigned(VLG_STATUS_NONFINITE));
-      if (tid < 2 * Kb) p.grad_omega[size_t(n) * 2 * Kb + tid] = g;
-      else if (tid < 2 * Kb + 2) p.grad_a[2 * n + tid - 2 * Kb] = g;
-      else p.grad_b[2 * n + tid - 2 * Kb - 2] = g;
-    } else if (GRAD && !gout && tid < 2 * Kb) {
-      const int k = tid >> 1, d = tid & 1;
-      const float tend = p.t[T - 1];
-      float P[MAX_KB];
-      design_row(tend, n_poly, Kb, s.basis, P);
-      const float2 ze = spline_point(tend, n_poly, s.coef, pa, pb);
-      const float err = d == 0 ? ze.x - pb.x : ze.y - pb.y;
-      const float g = s.gacc[tid] + (2.0f * p.penalty_w) * err * P[k];
-      AdamScalars sc = adam_scalars(p.step0 + step + 1, p.lr, p.beta1, p.beta2);
-      float om = s.om[tid], mm = s.om[2 * MAX_KB + tid], vv = s.om[4 * MAX_KB + tid];
-      adam_update(om, mm, vv, g, sc, p.one_minus_b1, p.beta2f, p.one_minus_b2, p.eps);
-      s.om[tid] = om;
-      s.om[2 * MAX_KB + tid] = mm;
-      s.om[4 * MAX_KB + tid] = vv;
-    }
+    // ---- step epilogue: energy out; gradient out, or penalty gradient and Adam ----
+    if (tid == 0) write_energy(p, n, step, e_tot, l_tot, status);
+    if (GOUT && tid < 2 * Kb + 4) write_grad(p, n, tid, tid < 2 * Kb ? s.gacc[tid] : gab[tid - 2 * Kb], status);
+    if (MODE == StepMode::Optimize && tid < 2 * Kb) penalty_adam_step(p, step, tid, s.gacc[tid], s.basis, s.coef, pa, pb, s.om);
     __syncthreads();
   }  // steps
 
-  if (GRAD && !gout && tid < 2 * Kb) {
-    p.omega[size_t(n) * 2 * Kb + tid] = s.om[tid];
-    p.adam_m[size_t(n) * 2 * Kb + tid] = s.om[2 * MAX_KB + tid];
-    p.adam_v[size_t(n) * 2 * Kb + tid] = s.om[4 * MAX_KB + tid];
-  }
+  if (MODE == StepMode::Optimize && tid < 2 * Kb) write_back(p, n, tid, s.om, status);
   __syncthreads();
   }  // curves of this CTA
   if (bad_draw) atomicOr(status, unsigned(VLG_STATUS_BAD_DRAW));
 }
 
-cudaError_t launch_simt(const StepParams& p, bool grad, cudaStream_t stream) {
+cudaError_t launch_simt(const StepParams& p, cudaStream_t stream) {
   const int W = simt_window_points(p.T, p.K, p.M);
   if (W < 2) return cudaErrorNotSupported;
   const size_t smem = simt_smem_bytes_w(W, p.K, p.M);
-  const int grid = simt_grid(p.N);
+  const int grid = persistent_grid(p.N);
   const int max_items = simt_max_items(W, p.K, p.M);
   if (p.workspace == nullptr || p.workspace_bytes < simt_workspace_bytes(p.N, p.T, p.K, p.M)) return cudaErrorInvalidValue;
   cudaError_t e = cudaMemsetAsync(p.workspace, 0, 256, stream);
@@ -612,8 +552,7 @@ cudaError_t launch_simt(const StepParams& p, bool grad, cudaStream_t stream) {
     kernel<<<grid, NTHREADS, smem, stream>>>(p, W, max_items);
     return cudaGetLastError();
   };
-  if (grad && p.grad_omega) return launch(simt_curve_kernel<true, true>);
-  return grad ? launch(simt_curve_kernel<true, false>) : launch(simt_curve_kernel<false, false>);
+  return with_mode(p.mode, [&](auto mode) { return launch(simt_curve_kernel<decltype(mode)::value>); });
 }
 
 }  // namespace vlg

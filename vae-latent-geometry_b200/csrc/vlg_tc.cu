@@ -361,11 +361,10 @@ static int tc_stages(int W, int K, int M, int xl2) {
   return int(nst);
 }
 
-// GOUT: gradient-output mode (vlg_curve_energy_grad, GRAD only): energy and dE/d(omega), dE/da, dE/db out, no Adam.
-// A template parameter, not a runtime branch, so that the optimiser's instantiations carry none of its code.
-template <bool GRAD, int FMT, bool XL2, bool GOUT>
+template <StepMode MODE, int FMT, bool XL2>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, int nst, int W, int G_) {
-  static_assert(GRAD || !GOUT, "gradient-output mode runs the backward items");
+  constexpr bool GRAD = MODE != StepMode::Energy;       // backward items
+  constexpr bool GOUT = MODE == StepMode::EnergyGrad;   // gradient out instead of Adam
   constexpr bool xl2 = XL2;               // left-end outputs / differences in the L2 workspace instead of shared memory
   constexpr int GM = XL2 ? TC_MAX_G : 1;  // curves per window this kernel is built for
   const int G = XL2 ? G_ : 1;             // curves per window of this launch: G > 1 = G whole curves (W = G T points)
@@ -702,7 +701,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
         if (j < Gcur) {
           const size_t o = size_t(n0 + j) * 2 * Kb + c;
           s.om[j * OM_STRIDE + c] = __ldcg(p.omega + o);
-          if (GRAD && !GOUT) {
+          if (MODE == StepMode::Optimize) {
             s.om[j * OM_STRIDE + 2 * MAX_KB + c] = __ldcg(p.adam_m + o);
             s.om[j * OM_STRIDE + 4 * MAX_KB + c] = __ldcg(p.adam_v + o);
           }
@@ -1423,57 +1422,26 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
           PH(15);
         }  // windows
 
-        if (t512 < Gcur) {
-          const int n = n0 + t512;
-          const float E = s.etot[2 * t512] / float(Mtot);
-          // fp16 operands overflow above 65504: inf/NaN reach the energy (forward) or omega (backward)
-          if (!(fabsf(E) <= 3.0e38f)) atomicOr(&queue[1], unsigned(VLG_STATUS_NONFINITE));
-          if (p.energy_trace) p.energy_trace[size_t(step) * p.N + n] = E;
-          if (step == p.steps - 1) {
-            if (p.energy_last) p.energy_last[n] = E;
-            if (p.length_out) p.length_out[n] = s.etot[2 * t512 + 1] / float(Mtot);
-          }
-        }
+        if (t512 < Gcur) write_energy(p, n0 + t512, step, s.etot[2 * t512], s.etot[2 * t512 + 1], &queue[1]);
         if (GOUT) {
-          // dE/d(omega), dE/da, dE/db of the energy alone
           const int ncol = 2 * Kb + 4;
           if (t512 < Gcur * ncol) {
-            const int j = t512 / ncol, c = t512 - j * ncol, n = n0 + j;
-            const float g = c < 2 * Kb ? s.gacc[j * 20 + c] : s.om[j * OM_STRIDE + 2 * MAX_KB + c - 2 * Kb];
-            if (!(fabsf(g) <= 3.0e38f)) atomicOr(&queue[1], unsigned(VLG_STATUS_NONFINITE));
-            if (c < 2 * Kb) p.grad_omega[size_t(n) * 2 * Kb + c] = g;
-            else if (c < 2 * Kb + 2) p.grad_a[2 * n + c - 2 * Kb] = g;
-            else p.grad_b[2 * n + c - 2 * Kb - 2] = g;
+            const int j = t512 / ncol, c = t512 - j * ncol;
+            write_grad(p, n0 + j, c, c < 2 * Kb ? s.gacc[j * 20 + c] : s.om[j * OM_STRIDE + 2 * MAX_KB + c - 2 * Kb],
+                       &queue[1]);
           }
-        } else if (GRAD && t512 < Gcur * 2 * Kb) {
+        } else if (MODE == StepMode::Optimize && t512 < Gcur * 2 * Kb) {
           const int j = t512 / (2 * Kb), c = t512 - j * 2 * Kb;
-          const int k = c >> 1, d = c & 1;
-          const float tend = p.t[T - 1];
-          float P[MAX_KB];
-          design_row(tend, n_poly, Kb, s.basis, P);
           const float* ab = s.pab + 4 * j;
-          const float2 pb = make_float2(ab[2], ab[3]);
-          const float2 ze = spline_point(tend, n_poly, s.coef + j * 64, make_float2(ab[0], ab[1]), pb);
-          const float err = d == 0 ? ze.x - pb.x : ze.y - pb.y;
-          const float g = s.gacc[j * 20 + c] + (2.0f * p.penalty_w) * err * P[k];
-          AdamScalars sc = adam_scalars(p.step0 + step + 1, p.lr, p.beta1, p.beta2);
-          float* o = s.om + j * OM_STRIDE;
-          float om = o[c], mm = o[2 * MAX_KB + c], vv = o[4 * MAX_KB + c];
-          adam_update(om, mm, vv, g, sc, p.one_minus_b1, p.beta2f, p.one_minus_b2, p.eps);
-          o[c] = om;
-          o[2 * MAX_KB + c] = mm;
-          o[4 * MAX_KB + c] = vv;
+          penalty_adam_step(p, step, c, s.gacc[j * 20 + c], s.basis, s.coef + j * 64, make_float2(ab[0], ab[1]),
+                            make_float2(ab[2], ab[3]), s.om + j * OM_STRIDE);
         }
         named_bar(3, EPI_THREADS);
       }  // steps
 
-      if (GRAD && !GOUT && t512 < Gcur * 2 * Kb) {
+      if (MODE == StepMode::Optimize && t512 < Gcur * 2 * Kb) {
         const int j = t512 / (2 * Kb), c = t512 - j * 2 * Kb;
-        const size_t o = size_t(n0 + j) * 2 * Kb + c;
-        p.omega[o] = s.om[j * OM_STRIDE + c];
-        p.adam_m[o] = s.om[j * OM_STRIDE + 2 * MAX_KB + c];
-        p.adam_v[o] = s.om[j * OM_STRIDE + 4 * MAX_KB + c];
-        if (!(fabsf(s.om[j * OM_STRIDE + c]) <= 3.0e38f)) atomicOr(&queue[1], unsigned(VLG_STATUS_NONFINITE));
+        write_back(p, n0 + j, c, s.om + j * OM_STRIDE, &queue[1]);
         __threadfence();
       }
       named_bar(3, EPI_THREADS);
@@ -1521,11 +1489,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
       const int chunk = int(unit / ngroups);
       const int step_lo = chunk * unit_steps, step_hi = min(p.steps, step_lo + unit_steps);
       // one weight set per window: per-curve sets (decoder_base) are only launched with G = 1
-      int dec_base = p.dec_base ? p.dec_base[n0] : 0;
-      if (dec_base < 0 || dec_base + K > p.K_total) {   // memory safety; reported through the status word
-        dec_base = 0;
-        if (lane == 0) atomicOr(&queue[1], unsigned(VLG_STATUS_BAD_PACKED));
-      }
+      const int dec_base = curve_dec_base(p, n0, lane == 0, &queue[1]);
       for (int step = step_lo; step < step_hi; ++step)
         for (int win = 0; win < nwin; ++win)
           for (int mb = 0; 2 * mb < Mtot; ++mb, ++wseq) {
@@ -1551,12 +1515,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
               if (p.draws != nullptr) {
                 for (int m = 0; m < Mb; ++m)
                   for (int role = 0; role < 2; ++role) {
-                    uint8_t v = 255;
-                    if (seg_ok) {
-                      v = p.draws[(((size_t(n) * p.steps + step) * Mtot + 2 * mb + m) * 2 + role) * size_t(T - 1) + seg0 + i];
-                      if (v >= K) { v = uint8_t(K - 1); bad_draw = true; }   // memory safety; reported through the status word
-                    }
-                    sel[4 * (pt + role) + 2 * m + role] = v;
+                    sel[4 * (pt + role) + 2 * m + role] = seg_ok ? explicit_draw(p.draws, p.steps, Mtot, T, K, n, step, 2 * mb + m, role, seg0 + i, bad_draw) : 255;
                   }
                 if (Mb < 2) { sel[4 * pt + 2] = 255; sel[4 * pt + 7] = 255; }
               } else {
@@ -1654,17 +1613,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_curve_kernel(StepParams p, i
   if (warp == 2) tmem_dealloc(tmem, 512);
 }
 
-static int tc_grid(int N) {
-  int dev = 0, sms = 148;
-  if (cudaGetDevice(&dev) == cudaSuccess) {
-    int v = 0;
-    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && v > 0) sms = v;
-  } else {
-    (void)cudaGetLastError();
-  }
-  return N < sms ? N : sms;
-}
-
 // Launch plan.  Window length: as few 128-row items per curve as possible.  A decoder is drawn by a point with
 // probability p = 1 - (1 - 1/K)^(2M); its row count n in a window of W points is ~Binomial(W, p) and it
 // costs ceil(n/128) items.  Evaluate the expected item count for every admissible number of windows, for both
@@ -1674,12 +1622,6 @@ static int tc_grid(int N) {
 struct TcPlan {
   int W, nst, xl2, G;   // W = points per window (all curves), G = curves per window
 };
-static double tc_expected_items(int w, double p) {
-  const double mean = w * p, sd = sqrt(w * p * (1.0 - p)) + 1e-9;
-  double items = 0.0;
-  for (int q = 0; q * 128 < w; ++q) items += 0.5 * erfc((q * 128 + 0.5 - mean) / (sd * 1.4142135623730951));  // P(n > 128 q)
-  return items;
-}
 static TcPlan tc_plan(int T, int K, int M, bool allow_multi) {
   if (M > TC_MAX_M) M = TC_MAX_M;   // samples per block
   const double p = 1.0 - pow(1.0 - 1.0 / K, 2.0 * M);
@@ -1702,7 +1644,7 @@ static TcPlan tc_plan(int T, int K, int M, bool allow_multi) {
       if (w <= TC_MAX_W && force_g <= 1) {
         const int nst = tc_stages(w, K, M, xl2);
         if (nst >= 2) {
-          double cost = nwin * (K * tc_expected_items(w, p) + 0.35);  // + per-window fixed cost in item units
+          double cost = nwin * (K * expected_items(w, p) + 0.35);  // + per-window fixed cost in item units
           if (nst == 2) cost *= 1.04;               // a two-stage weight ring cannot hold a whole GEMM's weights
           if (xl2) cost *= 1.45;
           if (cost < best_cost) { best_cost = cost; best = {w, nst, xl2, 1}; }
@@ -1717,7 +1659,7 @@ static TcPlan tc_plan(int T, int K, int M, bool allow_multi) {
         const int w = g * T;
         const int nst = tc_stages(w, K, M, 1);
         if (nst < 2) continue;
-        double cost = (K * tc_expected_items(w, p) + 0.35) / g * 1.45;
+        double cost = (K * expected_items(w, p) + 0.35) / g * 1.45;
         if (nst == 2) cost *= 1.04;
         if (cost < best_cost) { best_cost = cost; best = {w, nst, 1, g}; }
       }
@@ -1731,7 +1673,7 @@ size_t tc_workspace_bytes(int N, int T, int K, int M) {
   const TcPlan pl = tc_plan(T, K, M, true);   // the multi-curve plan needs at least as much as the single-curve one
   const TcPlan p1 = tc_plan(T, K, M, false);
   const size_t a = tc_ws_cta_words(K, M, pl.W), b = tc_ws_cta_words(K, M, p1.W);
-  return tc_queue_words(N) * 4 + size_t(tc_grid(N)) * (a > b ? a : b) * 4;
+  return tc_queue_words(N) * 4 + size_t(persistent_grid(N)) * (a > b ? a : b) * 4;
 }
 
 #ifdef VLG_TC_STATS
@@ -1743,7 +1685,7 @@ extern "C" int vlg_debug_tc_phase(long long* host_out, int n) {
 }
 #endif
 
-cudaError_t launch_tc(const StepParams& p, bool grad, cudaStream_t stream) {
+cudaError_t launch_tc(const StepParams& p, cudaStream_t stream) {
   if (p.precision < 1 || p.precision > 4) return cudaErrorNotSupported;
   const int fmt = p.precision == 1 ? FMT_TF32 : p.precision == 3 ? FMT_F16 : p.precision == 4 ? FMT_F16X3F : FMT_F16X3;
   if (p.K > TC_MAX_K || p.M < 1) return cudaErrorNotSupported;
@@ -1754,7 +1696,7 @@ cudaError_t launch_tc(const StepParams& p, bool grad, cudaStream_t stream) {
   if (p.workspace == nullptr || p.workspace_bytes < tc_workspace_bytes(p.N, p.T, p.K, p.M)) return cudaErrorInvalidValue;
   const size_t smem = tc_smem_fixed_bytes(W, p.K, Mc, xl2) + size_t(2) * nst * STAGE_BYTES;
   const int ngroups = (p.N + G - 1) / G;
-  const int grid = tc_grid(ngroups);
+  const int grid = persistent_grid(ngroups);
   StepParams q = p;
   // chunks of a curve (group) per launch: at least 4, and enough work units (~48 per CTA) that the last wave's
   // tail -- at most one unit -- stays a small fraction of the launch
@@ -1770,20 +1712,19 @@ cudaError_t launch_tc(const StepParams& p, bool grad, cudaStream_t stream) {
     kernel<<<grid, TC_THREADS, smem, stream>>>(q, nst, W, G);
     return cudaGetLastError();
   };
-  auto by_fmt = [&](auto grad_c, auto xl2_c, auto gout_c) -> cudaError_t {
-    constexpr bool G = decltype(grad_c)::value, X = decltype(xl2_c)::value, O = decltype(gout_c)::value;
-    if (fmt == FMT_TF32) return launch(tc_curve_kernel<G, FMT_TF32, X, O>);
-    if (fmt == FMT_F16) return launch(tc_curve_kernel<G, FMT_F16, X, O>);
-    if constexpr (G) {   // forward only: the mixed format IS the 3-term format
-      if (fmt == FMT_F16X3F) return launch(tc_curve_kernel<G, FMT_F16X3F, X, O>);
+  auto by_fmt = [&](auto mode_c, auto xl2_c) -> cudaError_t {
+    constexpr StepMode MODE = decltype(mode_c)::value;
+    constexpr bool X = decltype(xl2_c)::value;
+    if (fmt == FMT_TF32) return launch(tc_curve_kernel<MODE, FMT_TF32, X>);
+    if (fmt == FMT_F16) return launch(tc_curve_kernel<MODE, FMT_F16, X>);
+    if constexpr (MODE != StepMode::Energy) {   // forward only: the mixed format IS the 3-term format
+      if (fmt == FMT_F16X3F) return launch(tc_curve_kernel<MODE, FMT_F16X3F, X>);
     }
-    return launch(tc_curve_kernel<G, FMT_F16X3, X, O>);
+    return launch(tc_curve_kernel<MODE, FMT_F16X3, X>);
   };
-  using T_ = std::true_type;
-  using F_ = std::false_type;
-  if (grad && p.grad_omega) return xl2 ? by_fmt(T_{}, T_{}, T_{}) : by_fmt(T_{}, F_{}, T_{});
-  if (grad) return xl2 ? by_fmt(T_{}, T_{}, F_{}) : by_fmt(T_{}, F_{}, F_{});
-  return xl2 ? by_fmt(F_{}, T_{}, F_{}) : by_fmt(F_{}, F_{}, F_{});
+  return with_mode(p.mode, [&](auto mode_c) {
+    return xl2 ? by_fmt(mode_c, std::true_type{}) : by_fmt(mode_c, std::false_type{});
+  });
 }
 
 }  // namespace vlg

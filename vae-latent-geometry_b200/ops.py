@@ -84,6 +84,24 @@ def workspace_status(workspace: torch.Tensor) -> int:
     return flags.value
 
 
+def _step_args(packed, k_total, x_dim, k_active, n_poly, M, steps, a, b, omega, basis, t, draws, decoder_base, seed,
+               curve_id0, workspace):
+    """Checks the tensors the three step ops share.  Returns their C-ABI arguments in the runs the entry points
+    take them: (packed .. M), (a, b, omega), (basis .. curve_id0) and (workspace, its bytes, stream)."""
+    N, Kb = omega.shape[0], omega.shape[1]
+    T = t.shape[0]
+    if Kb != n_poly + 1:
+        raise _lib.VlgError(f"omega has Kb={Kb}, expected n_poly+1={n_poly + 1}")
+    head = [_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active, N, T, n_poly, M]
+    curve = [_chk(a, "a", shape=(N, 2)), _chk(b, "b", shape=(N, 2)), _chk(omega, "omega", shape=(N, Kb, 2))]
+    tail = [_chk(basis, "basis", shape=(4 * n_poly, Kb)), _chk(t, "t", shape=(T,)),
+            _chk(draws, "draws", dtype=torch.uint8, shape=(N, steps, M, 2, T - 1)),
+            _chk(decoder_base, "decoder_base", dtype=torch.int32, shape=(N,)), seed & 0xFFFFFFFFFFFFFFFF, curve_id0]
+    ws = [_chk(workspace, "workspace", dtype=torch.uint8), workspace.numel() if workspace is not None else 0,
+          _stream(omega)]
+    return head, curve, tail, ws
+
+
 @torch.library.custom_op("vlg::optimize_steps",
                          mutates_args=("omega", "adam_m", "adam_v", "energy_last", "energy_trace", "workspace"))
 def optimize_steps(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, n_poly: int, M: int, steps: int, step0: int,
@@ -94,22 +112,13 @@ def optimize_steps(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int
                    beta2: float, eps: float, penalty_w: float, energy_last: torch.Tensor,
                    energy_trace: Optional[torch.Tensor], precision: int,
                    workspace: Optional[torch.Tensor]) -> None:
-    N, Kb = omega.shape[0], omega.shape[1]
-    T = t.shape[0]
-    if Kb != n_poly + 1:
-        raise _lib.VlgError(f"omega has Kb={Kb}, expected n_poly+1={n_poly + 1}")
-    args = [_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active, N, T, n_poly, M, steps, step0,
-            _chk(a, "a", shape=(N, 2)), _chk(b, "b", shape=(N, 2)), _chk(omega, "omega", shape=(N, Kb, 2)),
-            _chk(adam_m, "adam_m", shape=(N, Kb, 2)), _chk(adam_v, "adam_v", shape=(N, Kb, 2)),
-            _chk(basis, "basis", shape=(4 * n_poly, Kb)), _chk(t, "t", shape=(T,)),
-            _chk(draws, "draws", dtype=torch.uint8, shape=(N, steps, M, 2, T - 1)) if draws is not None else 0,
-            _chk(decoder_base, "decoder_base", dtype=torch.int32, shape=(N,)) if decoder_base is not None else 0,
-            seed & 0xFFFFFFFFFFFFFFFF, curve_id0, lr, beta1, beta2, eps, penalty_w,
-            _chk(energy_last, "energy_last", shape=(N,)),
-            _chk(energy_trace, "energy_trace", shape=(steps, N)) if energy_trace is not None else 0,
-            precision,
-            _chk(workspace, "workspace", dtype=torch.uint8) if workspace is not None else 0,
-            workspace.numel() if workspace is not None else 0, _stream(omega)]
+    head, curve, tail, ws = _step_args(packed, k_total, x_dim, k_active, n_poly, M, steps, a, b, omega, basis, t, draws,
+                                       decoder_base, seed, curve_id0, workspace)
+    N = omega.shape[0]
+    args = [*head, steps, step0, *curve, _chk(adam_m, "adam_m", shape=omega.shape),
+            _chk(adam_v, "adam_v", shape=omega.shape), *tail, lr, beta1, beta2, eps, penalty_w,
+            _chk(energy_last, "energy_last", shape=(N,)), _chk(energy_trace, "energy_trace", shape=(steps, N)),
+            precision, *ws]
     with torch.cuda.device(omega.device):
         _lib.check(_lib.load().vlg_optimize_steps(*args), "vlg_optimize_steps")
 
@@ -120,19 +129,11 @@ def curve_energy(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, 
                  draws: Optional[torch.Tensor], decoder_base: Optional[torch.Tensor], seed: int, curve_id0: int, step: int,
                  energy: torch.Tensor, length: Optional[torch.Tensor], precision: int,
                  workspace: Optional[torch.Tensor]) -> None:
-    N, Kb = omega.shape[0], omega.shape[1]
-    T = t.shape[0]
-    if Kb != n_poly + 1:
-        raise _lib.VlgError(f"omega has Kb={Kb}, expected n_poly+1={n_poly + 1}")
-    args = [_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active, N, T, n_poly, M,
-            _chk(a, "a", shape=(N, 2)), _chk(b, "b", shape=(N, 2)), _chk(omega, "omega", shape=(N, Kb, 2)),
-            _chk(basis, "basis", shape=(4 * n_poly, Kb)), _chk(t, "t", shape=(T,)),
-            _chk(draws, "draws", dtype=torch.uint8, shape=(N, 1, M, 2, T - 1)) if draws is not None else 0,
-            _chk(decoder_base, "decoder_base", dtype=torch.int32, shape=(N,)) if decoder_base is not None else 0,
-            seed & 0xFFFFFFFFFFFFFFFF, curve_id0, step, _chk(energy, "energy", shape=(N,)),
-            _chk(length, "length", shape=(N,)) if length is not None else 0, precision,
-            _chk(workspace, "workspace", dtype=torch.uint8) if workspace is not None else 0,
-            workspace.numel() if workspace is not None else 0, _stream(omega)]
+    head, curve, tail, ws = _step_args(packed, k_total, x_dim, k_active, n_poly, M, 1, a, b, omega, basis, t, draws,
+                                       decoder_base, seed, curve_id0, workspace)
+    N = omega.shape[0]
+    args = [*head, *curve, *tail, step, _chk(energy, "energy", shape=(N,)), _chk(length, "length", shape=(N,)),
+            precision, *ws]
     with torch.cuda.device(omega.device):
         _lib.check(_lib.load().vlg_curve_energy(*args), "vlg_curve_energy")
 
@@ -144,20 +145,12 @@ def curve_energy_grad(packed: torch.Tensor, k_total: int, x_dim: int, k_active: 
                       draws: Optional[torch.Tensor], decoder_base: Optional[torch.Tensor], seed: int, curve_id0: int,
                       step: int, energy: torch.Tensor, grad_omega: torch.Tensor, grad_a: torch.Tensor,
                       grad_b: torch.Tensor, precision: int, workspace: Optional[torch.Tensor]) -> None:
-    N, Kb = omega.shape[0], omega.shape[1]
-    T = t.shape[0]
-    if Kb != n_poly + 1:
-        raise _lib.VlgError(f"omega has Kb={Kb}, expected n_poly+1={n_poly + 1}")
-    args = [_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active, N, T, n_poly, M,
-            _chk(a, "a", shape=(N, 2)), _chk(b, "b", shape=(N, 2)), _chk(omega, "omega", shape=(N, Kb, 2)),
-            _chk(basis, "basis", shape=(4 * n_poly, Kb)), _chk(t, "t", shape=(T,)),
-            _chk(draws, "draws", dtype=torch.uint8, shape=(N, 1, M, 2, T - 1)) if draws is not None else 0,
-            _chk(decoder_base, "decoder_base", dtype=torch.int32, shape=(N,)) if decoder_base is not None else 0,
-            seed & 0xFFFFFFFFFFFFFFFF, curve_id0, step, _chk(energy, "energy", shape=(N,)),
-            _chk(grad_omega, "grad_omega", shape=(N, Kb, 2)), _chk(grad_a, "grad_a", shape=(N, 2)),
-            _chk(grad_b, "grad_b", shape=(N, 2)), precision,
-            _chk(workspace, "workspace", dtype=torch.uint8) if workspace is not None else 0,
-            workspace.numel() if workspace is not None else 0, _stream(omega)]
+    head, curve, tail, ws = _step_args(packed, k_total, x_dim, k_active, n_poly, M, 1, a, b, omega, basis, t, draws,
+                                       decoder_base, seed, curve_id0, workspace)
+    N = omega.shape[0]
+    args = [*head, *curve, *tail, step, _chk(energy, "energy", shape=(N,)),
+            _chk(grad_omega, "grad_omega", shape=omega.shape), _chk(grad_a, "grad_a", shape=(N, 2)),
+            _chk(grad_b, "grad_b", shape=(N, 2)), precision, *ws]
     with torch.cuda.device(omega.device):
         _lib.check(_lib.load().vlg_curve_energy_grad(*args), "vlg_curve_energy_grad")
 
