@@ -130,7 +130,7 @@ int vlg_optimize_steps(const void* packed, int K, int X, int K_active, int N, in
                        float* energy_last, float* energy_trace, int precision,
                        void* workspace, size_t workspace_bytes, void* stream);
 
-/* Status of the last vlg_optimize_steps / vlg_curve_energy / vlg_curve_energy_grad launch that used `workspace`: copies the
+/* Status of the last vlg_optimize_steps / vlg_curve_energy / vlg_curve_energy_grad / vlg_decode* launch that used `workspace`: copies the
  * status word back and SYNCHRONISES `stream` (the only entry point that does).  *flags (host
  * pointer, may be NULL) receives the VLG_STATUS_* bits; returns VLG_OK when none is set, else
  * VLG_ERR_NUMERIC.  Replaces the finite-check a caller of the reference would do on `energy`
@@ -184,6 +184,29 @@ int vlg_curve_energy_grad(const void* packed, int K, int X, int K_active, int N,
  */
 int vlg_ensemble_std_norm(const void* packed, int K, int X, int K_active, int G, const float* grid,
                           float* out, void* stream);
+
+/* ---- decoder ensemble outputs and their input gradient ----------------------------------------
+ * x[k,p,:] = f_k(z[p]) for the first K_active decoders of `packed`: the reference's
+ *   torch.stack([d(z).mean for d in decoders])   (src/optimize.py:50, src/init_splines_ensemble.py:49,
+ *                                                 the decoder check at src/optimize.py:108-116)
+ * with f_k the 2 -> 128 -> ReLU -> 128 -> ReLU -> X MLP of src/train.py:80-85.  z [P,2], x [K_active,P,X], fp32,
+ * contiguous; offsets are 64-bit (K_active * P * X may exceed 2^31).
+ * vlg_decode_backward: dz[p] = sum_k W1^T (m1 . W2^T (m2 . W3^T dx[k,p])), the input gradient autograd forms for a
+ * loss on those outputs (no weight gradients).  dx [K_active,P,X], dz [P,2].  The ReLU masks m1, m2 are recomputed
+ * from z, so the two calls share no state.  The decoders are summed in a fixed order with no atomics: repeated calls
+ * give the same bits, and each point's dz does not depend on the other points.  Each row of dx is normalised by a power
+ * of two before it is rounded to a tensor-core operand, so the result scales exactly with dx.
+ * Precision: any VLG_PRECISION_*; the tensor-core ones need K_active <= 128 (VLG_ERR_UNSUPPORTED beyond).
+ * VLG_PRECISION_F16X3F runs the forward GEMMs as F16X3 and the backward GEMMs (B3, B2) single-term.
+ * workspace: VLG_DECODE_WORKSPACE_BYTES; vlg_workspace_status reads the launch's status (VLG_STATUS_BAD_PACKED,
+ * VLG_STATUS_NONFINITE for a non-finite z, x or dz component).  Asynchronous on `stream`; allocates nothing.
+ * Argument errors are returned before any CUDA call.
+ */
+#define VLG_DECODE_WORKSPACE_BYTES 256   /* status header read by vlg_workspace_status */
+int vlg_decode(const void* packed, int K, int X, int K_active, int P, const float* z, float* x,
+               int precision, void* workspace, size_t workspace_bytes, void* stream);
+int vlg_decode_backward(const void* packed, int K, int X, int K_active, int P, const float* z, const float* dx,
+                        float* dz, int precision, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- spline evaluation ----------------------------------------------------------------
  * z[T,N,2] = GeodesicSplineBatch.forward(t) (src/optimize.py:22-35).  Used by the drop-in

@@ -43,6 +43,10 @@ SIGNATURES = {
     "vlg_spline_points": (c_int, [c_int, c_int, c_int] + [c_void_p] * 7),
     "vlg_spline_points_backward": (c_int, [c_int, c_int, c_int] + [c_void_p] * 7),
     "vlg_fit_splines": (c_int, [c_int, c_int, c_int] + [c_void_p] * 6),
+    "vlg_decode": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,      # packed K X K_active P z x
+                           c_int, c_void_p, c_size_t, c_void_p]),
+    "vlg_decode_backward": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,  # .. z dx dz
+                                    c_int, c_void_p, c_size_t, c_void_p]),
 }
 
 

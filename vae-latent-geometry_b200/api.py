@@ -5,6 +5,7 @@ Same names and argument meaning as the reference where a counterpart exists:
   reference                                             here
   ---------------------------------------------------   -----------------------------------
   list(model.decoder)            (src/optimize.py:103)  DecoderEnsemble.from_state_dict(...)
+  torch.stack([d(z).mean for d in decoders]) (50)       decoders(z), differentiable in z
   GeodesicSplineBatch(a,b,basis,omega,n_poly)   (13-35)  GeodesicSplineBatch (same signature)
   compute_energy_mc(model, decoders, t_vals, M) (38-75)  compute_energy_mc (same signature, +draws/seed)
   loss.sum().backward()                           (161)  autograd through compute_energy_mc and
@@ -107,6 +108,28 @@ class DecoderEnsemble:
     def device(self):
         return self.packed.device
 
+    # ---- evaluation -------------------------------------------------------------------
+    def __call__(self, z: torch.Tensor, precision: Optional[str] = None, check: bool = True) -> torch.Tensor:
+        """Outputs of every active decoder at the latent points z [..., 2] (any float dtype): fp32 [K_active, ..., X],
+        ``torch.stack([d(z).mean for d in decoders])`` of the reference (src/optimize.py:50,
+        src/init_splines_ensemble.py:49).  E.g. ``decoders(model(t_vals))`` is its [K, T, N, X].
+
+        Differentiable in z: with grad mode on and z.requires_grad, the backward runs vlg_decode_backward
+        (dz = sum_k J_k(z)^T dx[k], no weight gradients, once differentiable).  precision=None is DEFAULT_PRECISION,
+        with the fallbacks of the step kernels (more than 128 decoders, or one decoder in 'tf32' / 'f16': the fp32
+        kernel).  check=True reads the status word back (one stream synchronisation) and raises VlgError on a
+        non-finite output or gradient or a packed buffer that does not match its K / X."""
+        if not isinstance(z, torch.Tensor) or not z.is_cuda:
+            raise _lib.VlgError("DecoderEnsemble(z): z must be a CUDA tensor (vlg_b200 has no CPU path)")
+        if z.dim() < 1 or z.shape[-1] != 2 or not z.is_floating_point():
+            raise _lib.VlgError(f"DecoderEnsemble(z): z must be a float tensor [..., 2], got {z.dtype} {tuple(z.shape)}")
+        prec = _resolve_precision(precision, self, 1)
+        if torch.is_grad_enabled() and z.requires_grad:
+            x = _Decode.apply(z, self, prec, check)
+        else:
+            x = _decode(self, z.detach().reshape(-1, 2).float().contiguous(), prec, check)
+        return x.reshape(len(self), *z.shape[:-1], self.X)
+
 
 def _refuse_untracked_grads(what: str, **tensors) -> None:
     """Gradients flow to omega, a and b only: refuse instead of leaving .grad of anything else at None."""
@@ -140,6 +163,50 @@ class _SplinePoints(torch.autograd.Function):
         gb = torch.empty_like(ga)
         ops.spline_points_backward(ctx.n_poly, basis, t, dz.contiguous().float(), go, ga, gb)
         return go, ga, gb, None, None, None
+
+
+def _decode(decoders: DecoderEnsemble, z: torch.Tensor, prec: int, check: bool) -> torch.Tensor:
+    """x [K_active, P, X] of the points z [P, 2] (fp32, contiguous)."""
+    x = torch.empty((len(decoders), z.shape[0], decoders.X), dtype=torch.float32, device=z.device)
+    if z.shape[0] == 0:
+        return x
+    ws = torch.empty(ops.DECODE_WORKSPACE_BYTES, dtype=torch.uint8, device=z.device)
+    ops.decode(decoders.packed, decoders.K, decoders.X, len(decoders), z, x, prec, ws)
+    if check:
+        _raise_on_status(ws, "DecoderEnsemble")
+    return x
+
+
+def _decode_backward(decoders: DecoderEnsemble, z: torch.Tensor, dx: torch.Tensor, prec: int, check: bool) -> torch.Tensor:
+    """dz [P, 2] = sum_k J_k(z)^T dx[k] for z [P, 2] and dx [K_active, P, X] (fp32, contiguous)."""
+    dz = torch.empty((z.shape[0], 2), dtype=torch.float32, device=z.device)
+    if z.shape[0] == 0:
+        return dz
+    ws = torch.empty(ops.DECODE_WORKSPACE_BYTES, dtype=torch.uint8, device=z.device)
+    ops.decode_backward(decoders.packed, decoders.K, decoders.X, len(decoders), z, dx, dz, prec, ws)
+    if check:
+        _raise_on_status(ws, "DecoderEnsemble backward")
+    return dz
+
+
+class _Decode(torch.autograd.Function):
+    """x = decoders(z); the backward recomputes the ReLU masks from z in vlg_decode_backward (no saved activations)."""
+
+    @staticmethod
+    def forward(ctx, z, decoders, prec, check):
+        zf = z.detach().reshape(-1, 2).float().contiguous()
+        ctx.save_for_backward(zf)
+        ctx.decoders, ctx.prec, ctx.check, ctx.z_shape, ctx.z_dtype = decoders, prec, check, z.shape, z.dtype
+        return _decode(decoders, zf, prec, check)
+
+    @staticmethod
+    def backward(ctx, dx):
+        # once differentiable: the kernel forms dz only, so a graph of the backward (create_graph=True) cannot exist
+        if torch.is_grad_enabled():
+            raise _lib.VlgError("DecoderEnsemble: double backward is not supported (dz is once differentiable)")
+        (zf,) = ctx.saved_tensors
+        dz = _decode_backward(ctx.decoders, zf, dx.float().contiguous(), ctx.prec, ctx.check)
+        return dz.reshape(ctx.z_shape).to(ctx.z_dtype), None, None, None
 
 
 class _CurveEnergy(torch.autograd.Function):

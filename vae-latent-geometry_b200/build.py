@@ -9,7 +9,7 @@ from pathlib import Path
 PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 LIB_PATH = PKG_DIR / "libvlg_b200.so"
-SOURCES = ["vlg_api.cu", "vlg_simt.cu", "vlg_pack.cu", "vlg_tc.cu"]
+SOURCES = ["vlg_api.cu", "vlg_simt.cu", "vlg_pack.cu", "vlg_tc.cu", "vlg_decode.cu"]
 # test-only kernels (tcgen05 building-block selftests, include/vlg_selftest.h): a separate library,
 # never loaded by the product path
 SELFTEST_LIB_PATH = PKG_DIR / "libvlg_b200_selftest.so"

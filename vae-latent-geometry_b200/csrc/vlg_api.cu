@@ -230,6 +230,42 @@ int vlg_ensemble_std_norm(const void* packed, int K, int X, int K_active, int G,
   return e == cudaSuccess ? VLG_OK : cuda_fail(e);
 }
 
+}  // extern "C"
+
+namespace {
+
+// What vlg_decode and vlg_decode_backward share: argument checks (before any CUDA call), the device check, the launch.
+int decode_entry(const void* packed, int K, int X, int K_active, int P, const float* z, const float* dx, float* x, float* dz,
+                 int precision, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!packed || !z || !(x || dz) || (dz && !dx) || !workspace || P <= 0 || K_active < 1 || K_active > K)
+    return VLG_ERR_INVALID_ARGUMENT;
+  if (precision < VLG_PRECISION_FP32 || precision > VLG_PRECISION_F16X3F) return VLG_ERR_INVALID_ARGUMENT;
+  if (vlg_packed_decoders_bytes(K, vlg::H, X) == 0) return VLG_ERR_INVALID_ARGUMENT;
+  if (precision != VLG_PRECISION_FP32 && K_active > 128) return VLG_ERR_UNSUPPORTED;
+  if (workspace_bytes < VLG_DECODE_WORKSPACE_BYTES) return VLG_ERR_WORKSPACE;
+  int rc = check_device();
+  if (rc != VLG_OK) return rc;
+  cudaError_t e = vlg::launch_decode(packed, K, X, K_active, P, z, dx, x, dz, precision, workspace,
+                                     static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? VLG_OK : cuda_fail(e);
+}
+
+}  // namespace
+
+extern "C" {
+
+int vlg_decode(const void* packed, int K, int X, int K_active, int P, const float* z, float* x, int precision,
+               void* workspace, size_t workspace_bytes, void* stream) {
+  if (!x) return VLG_ERR_INVALID_ARGUMENT;
+  return decode_entry(packed, K, X, K_active, P, z, nullptr, x, nullptr, precision, workspace, workspace_bytes, stream);
+}
+
+int vlg_decode_backward(const void* packed, int K, int X, int K_active, int P, const float* z, const float* dx,
+                        float* dz, int precision, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!dx || !dz) return VLG_ERR_INVALID_ARGUMENT;
+  return decode_entry(packed, K, X, K_active, P, z, dx, nullptr, dz, precision, workspace, workspace_bytes, stream);
+}
+
 int vlg_spline_points(int N, int T, int n_poly, const float* a, const float* b, const float* omega,
                       const float* basis, const float* t, float* z, void* stream) {
   if (!a || !b || !omega || !basis || !t || !z || N <= 0 || T <= 0 || n_poly < 1) return VLG_ERR_INVALID_ARGUMENT;

@@ -81,6 +81,9 @@ cudaError_t launch_spline_points(int N, int T, int n_poly, const float* a, const
                                  const float* basis, const float* t, float* z, cudaStream_t stream);
 cudaError_t launch_spline_points_backward(int N, int T, int n_poly, const float* basis, const float* t, const float* dz,
                                           float* grad_omega, float* grad_a, float* grad_b, cudaStream_t stream);
+// Decoder ensemble outputs (dz == nullptr) or their input gradient (x unused); vlg_decode.cu
+cudaError_t launch_decode(const void* packed, int K_total, int X, int K, int P, const float* z, const float* dx, float* x,
+                          float* dz, int precision, void* workspace, cudaStream_t stream);
 cudaError_t launch_fit_splines(int N, int Lmax, int n_poly, const float* targets, const int32_t* lens,
                                const float* basis, float* omega, float* ab, cudaStream_t stream);
 

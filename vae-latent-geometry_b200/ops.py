@@ -73,7 +73,7 @@ def workspace_counters(workspace: torch.Tensor):
 
 
 def workspace_status(workspace: torch.Tensor) -> int:
-    """VLG_STATUS_* flags of the last step-kernel launch that used `workspace` (synchronises the stream)."""
+    """VLG_STATUS_* flags of the last step-kernel or decode launch that used `workspace` (synchronises the stream)."""
     import ctypes
     flags = ctypes.c_int(0)
     with torch.cuda.device(workspace.device):
@@ -165,6 +165,33 @@ def ensemble_std_norm(packed: torch.Tensor, k_total: int, x_dim: int, k_active: 
                                                      _chk(grid, "grid", shape=(G, 2)),
                                                      _chk(out, "out", shape=(G,)), _stream(grid)),
                    "vlg_ensemble_std_norm")
+
+
+DECODE_WORKSPACE_BYTES = 256   # VLG_DECODE_WORKSPACE_BYTES
+
+
+@torch.library.custom_op("vlg::decode", mutates_args=("x", "workspace"))
+def decode(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, z: torch.Tensor, x: torch.Tensor,
+           precision: int, workspace: torch.Tensor) -> None:
+    P = z.shape[0]
+    with torch.cuda.device(z.device):
+        _lib.check(_lib.load().vlg_decode(_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active, P,
+                                          _chk(z, "z", shape=(P, 2)), _chk(x, "x", shape=(k_active, P, x_dim)),
+                                          precision, _chk(workspace, "workspace", dtype=torch.uint8), workspace.numel(),
+                                          _stream(z)), "vlg_decode")
+
+
+@torch.library.custom_op("vlg::decode_backward", mutates_args=("dz", "workspace"))
+def decode_backward(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, z: torch.Tensor, dx: torch.Tensor,
+                    dz: torch.Tensor, precision: int, workspace: torch.Tensor) -> None:
+    P = z.shape[0]
+    with torch.cuda.device(z.device):
+        _lib.check(_lib.load().vlg_decode_backward(_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim,
+                                                   k_active, P, _chk(z, "z", shape=(P, 2)),
+                                                   _chk(dx, "dx", shape=(k_active, P, x_dim)),
+                                                   _chk(dz, "dz", shape=(P, 2)), precision,
+                                                   _chk(workspace, "workspace", dtype=torch.uint8), workspace.numel(),
+                                                   _stream(z)), "vlg_decode_backward")
 
 
 @torch.library.custom_op("vlg::spline_points", mutates_args=("z",))
