@@ -130,7 +130,8 @@ int vlg_optimize_steps(const void* packed, int K, int X, int K_active, int N, in
                        float* energy_last, float* energy_trace, int precision,
                        void* workspace, size_t workspace_bytes, void* stream);
 
-/* Status of the last vlg_optimize_steps / vlg_curve_energy / vlg_curve_energy_grad / vlg_decode* launch that used `workspace`: copies the
+/* Status of the last vlg_optimize_steps / vlg_curve_energy / vlg_curve_energy_grad / vlg_decode* /
+ * vlg_expected_energy launch that used `workspace` (the word sits at the same place in every one): copies the
  * status word back and SYNCHRONISES `stream` (the only entry point that does).  *flags (host
  * pointer, may be NULL) receives the VLG_STATUS_* bits; returns VLG_OK when none is set, else
  * VLG_ERR_NUMERIC.  Replaces the finite-check a caller of the reference would do on `energy`
@@ -207,6 +208,26 @@ int vlg_decode(const void* packed, int K, int X, int K_active, int P, const floa
                int precision, void* workspace, size_t workspace_bytes, void* stream);
 int vlg_decode_backward(const void* packed, int K, int X, int K_active, int P, const float* z, const float* dx,
                         float* dz, int precision, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- expected ensemble curve energy ------------------------------------------------------------
+ * The M -> infinity limit of compute_energy_mc (src/optimize.py:38-75) for curves given as points z [T][N][2] (a
+ * spline's model(t_vals), a Dijkstra poly-line, ...): with x_k(t) = f_k(z_t) for the first K_active decoders,
+ *   energy[n] = sum_{t<T-1} E_{k,l} ||f_l(z_{t+1}) - f_k(z_t)||^2 = sum_t ||mu_{t+1} - mu_t||^2 + sum_t c_t V_t
+ *   mu_t = (1/K) sum_k x_k(t),  V_t = (1/K) sum_k ||x_k(t) - mu_t||^2,  c_t = 1 at the two ends, 2 inside,
+ * and, when grad_z is not NULL, grad_z[t][n] = dE_n/dz_t = (2/K) sum_k J_k(z_t)^T (c_t x_k(t) - mu_{t-1} - mu_{t+1})
+ * (only the neighbours that exist).  Three passes: every decoder's forward for the means, every decoder's forward
+ * again (and the backward for grad_z) for V_t and each point's energy term, and a fixed-order sum over t per curve.
+ * No atomics: repeated calls give the same bits, and a curve's energy and grad_z do not depend on the other curves.
+ * N >= 1, T >= 2, T * N <= INT_MAX; precision and the K_active / X limits as for vlg_decode; VLG_PRECISION_F16X3F
+ * runs the forward GEMMs 3-term and the backward GEMMs single-term.  workspace: at least
+ * vlg_expected_energy_workspace_bytes(N, T, X) bytes (the 256-byte status header, then mu [T*N*X] and the energy
+ * terms [T*N] floats; 0 for a shape outside the limits); vlg_workspace_status reads the launch's status
+ * (VLG_STATUS_BAD_PACKED, VLG_STATUS_NONFINITE for a non-finite z, mean, energy term, energy or grad_z component).
+ * Asynchronous on `stream`; allocates nothing.  Argument errors are returned before any CUDA call.
+ */
+size_t vlg_expected_energy_workspace_bytes(int N, int T, int X);
+int vlg_expected_energy(const void* packed, int K, int X, int K_active, int N, int T, const float* z, float* energy,
+                        float* grad_z, int precision, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- spline evaluation ----------------------------------------------------------------
  * z[T,N,2] = GeodesicSplineBatch.forward(t) (src/optimize.py:22-35).  Used by the drop-in

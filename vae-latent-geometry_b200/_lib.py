@@ -47,6 +47,9 @@ SIGNATURES = {
                            c_int, c_void_p, c_size_t, c_void_p]),
     "vlg_decode_backward": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,  # .. z dx dz
                                     c_int, c_void_p, c_size_t, c_void_p]),
+    "vlg_expected_energy_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "vlg_expected_energy": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p,   # packed K X K_active N T z
+                                    c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),  # energy grad_z ..
 }
 
 

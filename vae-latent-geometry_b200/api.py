@@ -11,6 +11,7 @@ Same names and argument meaning as the reference where a counterpart exists:
   loss.sum().backward()                           (161)  autograd through compute_energy_mc and
                                                            GeodesicSplineBatch.forward (omega, a, b)
   optim.Adam([omega], lr) + the step loop     (153-162)  optimize_splines(model, decoders, t_vals, steps, ...)
+  E over the draws of compute_energy_mc (M -> inf)       expected_curve_energy(decoders, model(t_vals)), differentiable
   compute_energy / compute_geodesic_lengths              compute_energy / compute_geodesic_lengths
      (src/single_decoder/optimize_energy_batched.py:42-57)
   construct_nullspace_basis      (optimize_energy.py:58)  construct_nullspace_basis
@@ -207,6 +208,66 @@ class _Decode(torch.autograd.Function):
         (zf,) = ctx.saved_tensors
         dz = _decode_backward(ctx.decoders, zf, dx.float().contiguous(), ctx.prec, ctx.check)
         return dz.reshape(ctx.z_shape).to(ctx.z_dtype), None, None, None
+
+
+def _expected_energy(decoders: DecoderEnsemble, z: torch.Tensor, prec: int, check: bool, grad: bool):
+    """(energy [N], dE/dz [T, N, 2] or None) of the curves z [T, N, 2] (fp32, contiguous)."""
+    T, N = z.shape[0], z.shape[1]
+    energy = torch.empty(N, dtype=torch.float32, device=z.device)
+    dz = torch.empty_like(z) if grad else None
+    if N == 0:
+        return energy, dz
+    ws = torch.empty(ops.expected_energy_workspace_bytes(N, T, decoders.X), dtype=torch.uint8, device=z.device)
+    ops.expected_energy(decoders.packed, decoders.K, decoders.X, len(decoders), z, energy, dz, prec, ws)
+    if check:
+        _raise_on_status(ws, "expected_curve_energy")
+    return energy, dz
+
+
+class _ExpectedEnergy(torch.autograd.Function):
+    """Expected energy [N] with the dE/dz one EnergyGrad launch formed next to it; the backward only scales dE/dz
+    by the incoming dL/dE[n]."""
+
+    @staticmethod
+    def forward(ctx, z, decoders, prec, check):
+        energy, dz = _expected_energy(decoders, z.detach().float().contiguous(), prec, check, grad=True)
+        ctx.save_for_backward(dz)
+        ctx.z_dtype = z.dtype
+        return energy
+
+    @staticmethod
+    def backward(ctx, grad_e):
+        # once differentiable: the kernel forms dE/dz only, so a graph of the backward (create_graph=True) cannot exist
+        if torch.is_grad_enabled():
+            raise _lib.VlgError("expected_curve_energy: double backward is not supported (dE/dz is once differentiable)")
+        (dz,) = ctx.saved_tensors
+        return (grad_e.to(torch.float32)[None, :, None] * dz).to(ctx.z_dtype), None, None, None
+
+
+def expected_curve_energy(decoders: DecoderEnsemble, z: torch.Tensor, precision: Optional[str] = None,
+                          check: bool = True) -> torch.Tensor:
+    """Expected ensemble energy [N] of the curves z [T, N, 2] (any float dtype): the M -> infinity limit of
+    compute_energy_mc (src/optimize.py:38-75), i.e. its expectation over independent uniform decoder pairs,
+        E_n = sum_t ||mu_{t+1} - mu_t||^2 + sum_t c_t V_t,
+    with mu_t / V_t the ensemble mean / variance of the decoder outputs at z_t and c_t the number of segments that
+    touch point t.  Deterministic: ``torch.sqrt(expected_curve_energy(decoders, model(t_vals)))`` is the length the
+    reference's MC value estimates.  z can be any point sequence (a spline's ``model(t_vals)``, a Dijkstra path).
+
+    Differentiable in z: with grad mode on and z.requires_grad, ONE launch also forms dE/dz (once differentiable); a
+    spline's omega, a and b get their gradients through model(t_vals).  precision=None is DEFAULT_PRECISION, with the
+    fallbacks of DecoderEnsemble.__call__.  check=True reads the status word back (one stream synchronisation) and
+    raises VlgError on a non-finite result or a packed buffer that does not match its K / X."""
+    if not isinstance(z, torch.Tensor) or z.dim() != 3 or z.shape[-1] != 2 or not z.is_floating_point():
+        raise _lib.VlgError(f"expected_curve_energy: z must be a float tensor [T, N, 2], got "
+                            f"{getattr(z, 'dtype', type(z))} {tuple(getattr(z, 'shape', ()))}")
+    if z.shape[0] < 2:
+        raise _lib.VlgError(f"expected_curve_energy: a curve needs T >= 2 points, got T = {z.shape[0]}")
+    if not z.is_cuda:
+        raise _lib.VlgError("expected_curve_energy: z must be a CUDA tensor (vlg_b200 has no CPU path)")
+    prec = _resolve_precision(precision, decoders, 1)
+    if torch.is_grad_enabled() and z.requires_grad:
+        return _ExpectedEnergy.apply(z, decoders, prec, check)
+    return _expected_energy(decoders, z.detach().float().contiguous(), prec, check, grad=False)[0]
 
 
 class _CurveEnergy(torch.autograd.Function):

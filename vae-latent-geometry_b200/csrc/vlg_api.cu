@@ -1,6 +1,7 @@
 // extern "C" front end: argument validation, device check, dispatch.  See include/vlg.h.
 #include "../../include/vlg.h"
 
+#include <limits.h>
 #include <math.h>
 #include <stdio.h>
 
@@ -264,6 +265,28 @@ int vlg_decode_backward(const void* packed, int K, int X, int K_active, int P, c
                         float* dz, int precision, void* workspace, size_t workspace_bytes, void* stream) {
   if (!dx || !dz) return VLG_ERR_INVALID_ARGUMENT;
   return decode_entry(packed, K, X, K_active, P, z, dx, nullptr, dz, precision, workspace, workspace_bytes, stream);
+}
+
+size_t vlg_expected_energy_workspace_bytes(int N, int T, int X) {
+  if (N < 1 || T < 2 || X < 1 || X > 52 || size_t(T) * size_t(N) > size_t(INT_MAX)) return 0;
+  const size_t P = size_t(T) * size_t(N);
+  return VLG_DECODE_WORKSPACE_BYTES + (P * size_t(X) + P) * sizeof(float);
+}
+
+int vlg_expected_energy(const void* packed, int K, int X, int K_active, int N, int T, const float* z, float* energy,
+                        float* grad_z, int precision, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!packed || !z || !energy || !workspace || N < 1 || T < 2 || K_active < 1 || K_active > K)
+    return VLG_ERR_INVALID_ARGUMENT;
+  if (size_t(T) * size_t(N) > size_t(INT_MAX)) return VLG_ERR_INVALID_ARGUMENT;
+  if (precision < VLG_PRECISION_FP32 || precision > VLG_PRECISION_F16X3F) return VLG_ERR_INVALID_ARGUMENT;
+  if (vlg_packed_decoders_bytes(K, vlg::H, X) == 0) return VLG_ERR_INVALID_ARGUMENT;
+  if (precision != VLG_PRECISION_FP32 && K_active > 128) return VLG_ERR_UNSUPPORTED;
+  if (workspace_bytes < vlg_expected_energy_workspace_bytes(N, T, X)) return VLG_ERR_WORKSPACE;
+  int rc = check_device();
+  if (rc != VLG_OK) return rc;
+  cudaError_t e = vlg::launch_expected_energy(packed, K, X, K_active, N, T, z, energy, grad_z, precision, workspace,
+                                              static_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? VLG_OK : cuda_fail(e);
 }
 
 int vlg_spline_points(int N, int T, int n_poly, const float* a, const float* b, const float* omega,

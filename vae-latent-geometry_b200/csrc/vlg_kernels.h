@@ -84,6 +84,10 @@ cudaError_t launch_spline_points_backward(int N, int T, int n_poly, const float*
 // Decoder ensemble outputs (dz == nullptr) or their input gradient (x unused); vlg_decode.cu
 cudaError_t launch_decode(const void* packed, int K_total, int X, int K, int P, const float* z, const float* dx, float* x,
                           float* dz, int precision, void* workspace, cudaStream_t stream);
+// Expected ensemble curve energy of the curves z [T][N][2] and, if grad_z is not null, dE_n/dz; vlg_decode.cu.
+// workspace: the 256-byte status header, then mu [T*N*X] and e [T*N] floats (vlg_expected_energy_workspace_bytes)
+cudaError_t launch_expected_energy(const void* packed, int K_total, int X, int K, int N, int T, const float* z,
+                                   float* energy, float* grad_z, int precision, void* workspace, cudaStream_t stream);
 cudaError_t launch_fit_splines(int N, int Lmax, int n_poly, const float* targets, const int32_t* lens,
                                const float* basis, float* omega, float* ab, cudaStream_t stream);
 

@@ -106,6 +106,23 @@ __device__ __forceinline__ void tmem_ld32x2_sync(uint32_t taddr0, uint32_t taddr
       : "r"(taddr0), "r"(taddr1)
       : "memory");
 }
+__device__ __forceinline__ void tmem_ld8_sync(uint32_t taddr, uint32_t (&v)[8]) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];\n\t"
+      "tcgen05.wait::ld.sync.aligned;"
+      : VLG_R8(v, 0)
+      : "r"(taddr)
+      : "memory");
+}
+__device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t (&v)[4]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]),
+               "r"(v[3])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), VLG_W8(v, 0)
+               : "memory");
+}
 __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),

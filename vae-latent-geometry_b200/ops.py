@@ -194,6 +194,27 @@ def decode_backward(packed: torch.Tensor, k_total: int, x_dim: int, k_active: in
                                                    _stream(z)), "vlg_decode_backward")
 
 
+def expected_energy_workspace_bytes(N: int, T: int, X: int) -> int:
+    n = _lib.load().vlg_expected_energy_workspace_bytes(N, T, X)
+    if n == 0:
+        raise _lib.VlgError(f"unsupported expected-energy shape N={N} T={T} X={X} (need N >= 1, T >= 2, T*N < 2^31, X <= 52)")
+    return n
+
+
+@torch.library.custom_op("vlg::expected_energy", mutates_args=("energy", "grad_z", "workspace"))
+def expected_energy(packed: torch.Tensor, k_total: int, x_dim: int, k_active: int, z: torch.Tensor,
+                    energy: torch.Tensor, grad_z: Optional[torch.Tensor], precision: int,
+                    workspace: torch.Tensor) -> None:
+    T, N = z.shape[0], z.shape[1]
+    with torch.cuda.device(z.device):
+        _lib.check(_lib.load().vlg_expected_energy(_chk(packed, "packed", dtype=packed.dtype), k_total, x_dim, k_active,
+                                                   N, T, _chk(z, "z", shape=(T, N, 2)),
+                                                   _chk(energy, "energy", shape=(N,)),
+                                                   _chk(grad_z, "grad_z", shape=(T, N, 2)), precision,
+                                                   _chk(workspace, "workspace", dtype=torch.uint8), workspace.numel(),
+                                                   _stream(z)), "vlg_expected_energy")
+
+
 @torch.library.custom_op("vlg::spline_points", mutates_args=("z",))
 def spline_points(n_poly: int, a: torch.Tensor, b: torch.Tensor, omega: torch.Tensor, basis: torch.Tensor,
                   t: torch.Tensor, z: torch.Tensor) -> None:
